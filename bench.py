@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — IRFD train-step throughput on B200 (BASELINE.json metric: IRFD train samples/sec @256^2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--batch B] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A step = one generator training step of the reference (train.py:186-210 restricted to the differentiable losses,
@@ -12,6 +12,12 @@ random-init weights (seed 0).  Prints ONE JSON line on rank 0.
 
 --impl reference: the CPU restatement of the reference (oracle/irfd_oracle.py, "port": the reference itself is Python
 and does not travel to the GPU box) running the same step on the host cores, on a bounded sample.
+
+--dump-outputs DIR (native arm, rank 0): after the timed steps, what the last timed step computed is written as
+DIR/<name>.npy, so that two builds run with the same arguments (same seeded inputs and weights) can be compared output
+for output.  train: the step's loss, Gd's parameters after the Adam update and its gradients, every encoder stage's
+gradients and the encoders' BatchNorm running statistics; gen_infer / infer512: the generated images; d_step: the loss,
+its three terms, D's parameters after the update and its gradients.
 """
 from __future__ import annotations
 
@@ -59,7 +65,13 @@ def parse_args():
     ap.add_argument("--no-graph", action="store_true", help="the step's launch sequence launched kernel by kernel "
                     "instead of as one CUDA graph (profiling: ncu lists the same kernels the graph replays)")
     ap.add_argument("--cpu-sample", type=int, default=8, help="pairs per CPU-baseline step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step computed as "
+                    "DIR/<name>.npy (float32 / float64, a fixed seeded sample of large arrays, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs (--impl native)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.global_batch:
         if args.global_batch % world:
@@ -68,6 +80,34 @@ def parse_args():
     if not args.batch:
         args.batch = CONFIGS[args.config]["batch"]
     return args
+
+
+DUMP_MAX_ELEMENTS = 1 << 21   # per array; a larger one is written as a sample of about this many elements
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 20240229
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor as out_dir/<name>.npy: float64 stays float64, every other dtype becomes float32.  A tensor of
+    more than DUMP_MAX_ELEMENTS elements is flattened and sampled at sorted indices drawn from DUMP_SEED, so runs with
+    the same arguments sample the same positions."""
+    import numpy as np
+    import torch
+
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMENTS,), generator=g).unique()
+            t = t.reshape(-1)[idx.to(t.device)]
+        out[name] = (t if t.dtype == torch.float64 else t.float()).cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -298,7 +338,8 @@ def run_reference(args):
         return
     cfg = CONFIGS[args.config]
     units = CPU_UNITS[args.config]
-    val, done, threads, dt = cpu_arm(args.config, units, args.steps, args.warmup, budget_s=280.0)
+    # no time budget: every one of the --steps steps is timed
+    val, done, threads, dt = cpu_arm(args.config, units, args.steps, args.warmup, budget_s=float("inf"))
     line = {
         "impl": "reference", "metric": cfg["metric"], "value": val, "unit": cfg["unit"], "n_gpus": args.gpus,
         "steps": done, "warmup": args.warmup, "ms_per_step": 1e3 * dt / max(done, 1), "higher_is_better": True,
@@ -499,6 +540,14 @@ def run_native(args):
     e1.record()
     barrier()
     ms_e2e = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:   # before the passes below move the parameters again
+        from speak_hack_b200.trainer import STAGES
+
+        arrays = {"loss": loss, "gd_params": trainer.flat, "gd_grads": trainer.gflat}
+        arrays.update({f"encoder_grads_stage{k}": trainer.stage_flats[k] for k in STAGES})
+        arrays["encoder_bn_buffers"] = torch.cat([b.reshape(-1).float() for e in trainer.encoders
+                                                  for b in e.buffers() if b.is_floating_point()])
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- N > 1: on-hardware check of the exchange (reference semantics: DDP averages the per-rank gradients,
     # train.py:399-401).  One step through the captured graph WITH its NCCL buckets, then — from the same parameters,
@@ -621,6 +670,7 @@ def run_native_infer(args):
         eager = lambda: dstep.step(*dev_in)                                # noqa: E731
         runner = lambda a, b: dstep.step(a, b)                            # noqa: E731  (eager launches: no graph)
         pick = lambda out: [out.reshape(1)]                                # noqa: E731
+        names = ["loss"]
     elif args.config == "gen_infer":
         model = P.StyleGenerator(input_dim=6144).to(dev).eval()
         host_in = [(torch.randn(B, 6144, generator=g).abs() * 0.5).pin_memory()]
@@ -628,6 +678,7 @@ def run_native_infer(args):
         eager = lambda: model(*dev_in)                                     # noqa: E731
         runner = GraphedCall(lambda f: model(f), dev_in) if not args.no_graph else None
         pick = lambda out: [out]                                           # noqa: E731
+        names = ["images"]
     else:
         model = P.IRFD()
         model.Gd.synthesis = P.SynthesisNetwork(resolution=512)            # BASELINE config 5 / SURVEY Q9
@@ -644,6 +695,7 @@ def run_native_infer(args):
         eager = lambda: model(*dev_in)                                     # noqa: E731
         runner = IRFDInference(model, *dev_in) if not args.no_graph else None
         pick = lambda out: [out[0], out[1]]                                # noqa: E731
+        names = ["x_s_recon", "x_t_recon"]
     torch.manual_seed(11)
 
     def step(inputs):
@@ -738,6 +790,12 @@ def run_native_infer(args):
     barrier()
     ms_e2e = max_over_ranks(e0.elapsed_time(e1))
     checksum = float(host_out[(args.steps - 1) & 1][0].double().abs().mean())
+    if args.dump_outputs and rank == 0:
+        arrays = dict(zip(names, host_out[(args.steps - 1) & 1]))
+        if args.config == "d_step":
+            arrays.update(zip(("loss_real", "loss_fake", "r1"), dstep.last))
+            arrays.update(d_params=dstep.flat, d_grads=dstep.gflat)
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- roofline pass: eager launches, per-launch CUDA events around every tensor-core GEMM (one stream)
     ops.use_side_stream = False
