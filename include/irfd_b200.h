@@ -50,10 +50,22 @@ const char* irfd_last_error(void);
  *   mode 2: z = acc + bias[c] + nw[c]*noise[pixel]; a = lrelu(z, 0.2); y = a*sp1[b,c] + s1[b,c]
  *           noise [n*h*w] fp32, sp1/s1 [n][cout] fp32 (sp1 = style0 + 1)
  *   force_block_n: 0 = heuristic, else 64/128/256.
- * Shape rules: cin % 64 == 0, cout % 64 == 0; for ksize 3: w a power of two (<=128) or a multiple of 128, and
- * 128 pixels must form whole rows / whole images.
+ * Shape rules: cin % 64 == 0, cout % 64 == 0.  Two pixel-tile geometries (irfd_conv_gemm_geometry says which one a
+ * shape gets):
+ *   linear: 128 consecutive NHWC pixels are one tile — every pointwise conv of >= 128 pixels (ragged last tile), and
+ *           3x3 convs whose w divides 128 or is a multiple of 128 with 128 pixels forming whole rows / whole images.
+ *           Every mode.  With wgroups > 1 each group must cover a whole number of 128-pixel tiles.
+ *   boxed : every other shape (any n, h, w >= 1): a tile is a box of tw x th x tn <= 128 output pixels (w < 128:
+ *           tw = w, th = min(h, 128 / w), whole images per box when th == h; w > 128: 128-pixel row segments).
+ *           Modes 0 (plain) and 3 (affine) only — the eval-mode encoders' modes; the others return
+ *           IRFD_ERR_INVALID_ARGUMENT.  With wgroups > 1 the image count must split evenly into the groups (3x3 only).
  */
 int irfd_conv_gemm_m_tiles(int n, int h, int w);
+/* Host-only tile-geometry query (no CUDA call): out_host[7] = {boxed (0 linear / 1 boxed), tw, th, tn, tiles_w,
+ * tiles_h, tiles_n}; the launch has tiles_w * tiles_h * tiles_n pixel tiles (== irfd_conv_gemm_m_tiles when linear).
+ * Boxed tiles are ordered image-major, then rows, then columns.  Returns IRFD_ERR_INVALID_ARGUMENT for shapes neither
+ * geometry serves. */
+int irfd_conv_gemm_geometry(int n, int h, int w, int ksize, int wgroups, int* out_host);
 int irfd_conv_gemm(const void* x, int n, int h, int w, int cin, const void* wk, int cout, int ksize, void* out,
                    void* out2, int mode, const float* bias, const float* nw, const float* noise, const float* sp1,
                    const float* s1, float* stat_sum, float* stat_sq, int force_block_n, irfd_stream_t stream);
@@ -69,7 +81,7 @@ int irfd_conv_gemm_style_split(const void* x, int n, int h, int w, int cin, cons
 /* Grouped launches: the three ResNet-50 encoders of IRFD (model.py:33-35, 84-90) run the same layer shapes on the same
  * images with different weights, so one launch per layer serves all three.  wk stacks `wgroups` weight sets along its
  * rows ([wgroups*cout][k*k*cin]); the n images are split evenly, group-major ([wgroups][n/wgroups] images); each
- * group must cover a whole number of 128-pixel tiles.  a_shared != 0 (ksize 1 only): x holds one group's rows and is
+ * group must cover whole tiles (see the shape rules above).  a_shared != 0 (ksize 1 only): x holds one group's rows and is
  * read by every group (the stem's im2col matrix).  mode 0 (plain) or 1 (stats; partials stay [m_tiles][cout]).
  * The affine variant takes scale/shift as [wgroups][cout]. */
 int irfd_conv_gemm_grouped(const void* x, int n, int h, int w, int cin, const void* wk, int cout, int ksize, void* out,
@@ -195,8 +207,10 @@ int irfd_bn_backward_finish_sets(const void* g, const void* z, const float* mean
  * Layout / gather kernels for the strided ResNet convs and pooling (torchvision resnet.py:197-205, 133-137, 241).
  *   irfd_pack_conv_weight: fp32 OIHW -> bf16 GEMM operand. mode 0 fprop [o][tap][i]; 1 dgrad [i][flip(tap)][o];
  *                          2 dcol [(tap,i)][o]; 3 flat [o][kpad] (stem, k = c*49+kh*7+kw, zero padded).
- *   irfd_im2col_stem     : x NCHW fp32 [n,3,h,w] -> col [n*h/2*w/2][kpad] bf16 (7x7, stride 2, pad 3).
+ *   irfd_im2col_stem     : x NCHW fp32 [n,3,h,w] -> col [n*ho*wo][kpad] bf16 (7x7, stride 2, pad 3), w <= 579.
  *   irfd_im2col_3x3s2 / irfd_col2im_3x3s2: 3x3 stride-2 pad-1 gather [pix][tap*c + ch] and its adjoint.
+ *   The forward gathers (stem, 3x3/2, 1x1/2, max pool) take any h, w and produce ceil(h/2) x ceil(w/2) outputs
+ *   (torchvision's sizes); the adjoints (col2im, scatter_add, maxpool_bwd) need even h, w.
  *   irfd_subsample2 / irfd_scatter_add_s2: 1x1 stride-2 gather; adjoint fused with an add (a may be NULL).
  *   irfd_maxpool_fwd/bwd : MaxPool2d(3,2,1) with uint8 argmax taps (first maximum, like ATen).
  *   irfd_avgpool_fwd/bwd : AdaptiveAvgPool2d(1): [n,hw,c] bf16 <-> [n,c] fp32.

@@ -13,6 +13,8 @@
 //   running concurrently share A tiles in L2).
 // * conv_halo_kernel (further down) is the variant for 3x3 convs on rows of >= 128 pixels: one halo tile per
 //   64-channel chunk serves all nine taps.
+// * Shapes whose 128 consecutive pixels are not one TMA box (3x3 at 56^2, 28^2, 14^2, 7^2, odd sizes) run the
+//   box-tiled instances (conv_gemm_kernel<..., BOX = true>, PLAIN / AFFINE): a tile is a box of <= 128 pixels.
 //
 // Epilogue modes
 //   PLAIN : y = acc (+ bias[n])                                       -> bf16           (dgrad, 1x1, generic)
@@ -69,6 +71,10 @@ struct ConvGemmArgs {
   const float* bn_beta[4];
   int sg_tiles;               // m tiles per statistic group
   int warp_epi;               // non-STYLE modes of conv_gemm_kernel: per-warp epilogue (epilogue_tile_warp)
+  // Box-tiled geometry (conv_gemm_kernel<..., BOX = true>): m tile t is the TMA box of box_tw x box_th x box_tn output
+  // pixels at column tile t % box_tiles_w, row tile (t / box_tiles_w) % box_tiles_h, image tile t / (tiles_w * tiles_h)
+  // (see irfd_conv_gemm_geometry).  Unused by the linear geometry.
+  int box_tw, box_th, box_tn, box_tiles_w, box_tiles_h;
 };
 
 constexpr int kNumThreads = 320;      // 10 warps
@@ -90,17 +96,41 @@ struct GemmCfg {
   static constexpr uint32_t TMEM_COLS = (2 * BLOCK_N <= 128) ? 128 : (2 * BLOCK_N <= 256 ? 256 : 512);
 };
 
+// Box-tiled geometry: first output pixel (column, row, image) of m tile `m_tile`.
+__device__ __forceinline__ void box_origin(const ConvGemmArgs& p, int m_tile, int& w0, int& h0, int& n0) {
+  const int t = m_tile / p.box_tiles_w;
+  w0 = (m_tile - t * p.box_tiles_w) * p.box_tw;
+  h0 = (t % p.box_tiles_h) * p.box_th;
+  n0 = (t / p.box_tiles_h) * p.box_tn;
+}
+
+// Box-tiled geometry: flat NHWC pixel of row r of the tile whose origin is (w0, h0, n0), or -1 when the row lies past
+// the box (r >= tw * th * tn: stale A rows) or outside the tensor (a partial last tile, which the TMA store clips).
+__device__ __forceinline__ int box_pixel(const ConvGemmArgs& p, int w0, int h0, int n0, int r) {
+  const int wi = r % p.box_tw;
+  const int t = r / p.box_tw;
+  const int hi = t % p.box_th;
+  const int ni = t / p.box_th;
+  const int w = w0 + wi, h = h0 + hi, n = n0 + ni;
+  if (ni >= p.box_tn || w >= p.W || h >= p.H || n >= p.B) return -1;
+  return (n * p.H + h) * p.W + w;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Epilogue of ONE 128-row accumulator (TMEM columns [acc_col, acc_col + BLOCK_N)) whose first output row is the flat
 // pixel m0: TMEM -> registers -> fused math -> swizzled smem staging -> TMA store (+ STATS partials).
 // Called by the 8 epilogue warps (threads 64..319).  NBUF = staging buffers per output (1 or 2).
 // `release_bar`: arrived on (one lane per warp) as soon as the accumulator has been drained into registers.
+// BOX (PLAIN / AFFINE only): m0 = m tile * 128 of the box-tiled geometry; the first tw*th*tn staging rows are the box in
+// TMA order and go out as ONE 4-D store box (map_out is the 4-D [N][H][W][Cout] map), which clips rows outside the
+// tensor; the residual is read at each row's own pixel.
 // ------------------------------------------------------------------------------------------------
-template <int BLOCK_N, int MODE, int NBUF>
+template <int BLOCK_N, int MODE, int NBUF, bool BOX = false>
 __device__ __forceinline__ void epilogue_acc(const ConvGemmArgs& p, const CUtensorMap* map_out,
                                              const CUtensorMap* map_out2, uint32_t tmem_base, uint32_t acc_col,
                                              int m0, int n_tile, uint64_t* release_bar, uint8_t* stg_base, float* vec,
                                              uint32_t& chunk_counter) {
+  static_assert(!BOX || MODE == EPI_PLAIN || MODE == EPI_AFFINE, "the box-tiled geometry serves PLAIN / AFFINE only");
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int e = warp - 2;
@@ -117,6 +147,11 @@ __device__ __forceinline__ void epilogue_acc(const ConvGemmArgs& p, const CUtens
   const int pg0 = (m_tile / p.wg_tiles) * p.N_total + ng0;  // first channel of this tile in the per-group vectors
   float noise_r = 0.f;
   int img_local = 0;
+  int bw0 = 0, bh0 = 0, bn0 = 0, box_row = -1;  // BOX: tile origin and this thread's output pixel
+  if constexpr (BOX) {
+    box_origin(p, m_tile, bw0, bh0, bn0);
+    box_row = box_pixel(p, bw0, bh0, bn0, r);
+  }
   if constexpr (MODE == EPI_STYLE) {
     const int nimg = p.HW < 128 ? 128 / p.HW : 1;
     const int b0 = m0 / p.HW;
@@ -188,8 +223,9 @@ __device__ __forceinline__ void epilogue_acc(const ConvGemmArgs& p, const CUtens
       float o[8], o2[8];
       float rres[8];
       if constexpr (MODE == EPI_AFFINE) {
-        if (p.res != nullptr && m0 + r < p.M_total) {
-          const uint4 u = *reinterpret_cast<const uint4*>(p.res + (size_t)(m0 + r) * p.N_total + ng0 + cbase + jj * 8);
+        if (p.res != nullptr && (BOX ? box_row >= 0 : m0 + r < p.M_total)) {
+          const uint4 u = *reinterpret_cast<const uint4*>(p.res + (size_t)(BOX ? box_row : m0 + r) * p.N_total + ng0 +
+                                                          cbase + jj * 8);
           const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
           rres[0] = a0.x; rres[1] = a0.y; rres[2] = a1.x; rres[3] = a1.y;
           rres[4] = a2.x; rres[5] = a2.y; rres[6] = a3.x; rres[7] = a3.y;
@@ -316,7 +352,8 @@ __device__ __forceinline__ void epilogue_acc(const ConvGemmArgs& p, const CUtens
     if (warp == 2) {
       __syncwarp();
       if (elect_one_sync()) {
-        tma_store_2d(map_out, stg0, ng0 + chunk * 64, m0);
+        if constexpr (BOX) tma_store_4d(map_out, stg0, ng0 + chunk * 64, bw0, bh0, bn0);
+        else tma_store_2d(map_out, stg0, ng0 + chunk * 64, m0);
         if constexpr (MODE == EPI_STYLE) tma_store_2d(map_out2, stg1, ng0 + chunk * 64, m0);
         tma_store_commit();
       }
@@ -565,7 +602,13 @@ __device__ __forceinline__ void epilogue_tile_warp(const ConvGemmArgs& p, const 
 // MMA2 (with CL = 2): the pair executes 2-SM MMAs (tcgen05 cta_group::2, M = 256): each CTA loads ONLY its half of the
 // weight tile (its SM ingests A 16 KB + B 16 KB per k-block instead of 16 + 32), the leader's MMA warp issues for both,
 // commits go to both CTAs' barriers, both CTAs' epilogue warps release the accumulator at the leader.
-template <int BLOCK_N, int MODE, int CL = 1, bool MMA2 = false>
+//
+// BOX: the box-tiled geometry for 3x3 layers whose 128 consecutive pixels are not one TMA box (W neither dividing 128 nor
+// a multiple of it, or H not fitting whole boxes: 56^2, 28^2, 14^2, 7^2, odd sizes).  An m tile is a box of
+// P = tw*th*tn <= 128 pixels (see irfd_conv_gemm_geometry); every tap loads that box shifted by the tap offset, the
+// out-of-bounds zero fill is the padding as before.  A rows P..127 keep stale shared memory: MMA rows are independent,
+// so they only reach accumulator rows that are never stored.  M stays 128.  Single CTA, lockstep epilogue.
+template <int BLOCK_N, int MODE, int CL = 1, bool MMA2 = false, bool BOX = false>
 __global__ void __launch_bounds__(kNumThreads, 1)
 conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                  const __grid_constant__ CUtensorMap map_out, const __grid_constant__ CUtensorMap map_out2,
@@ -574,6 +617,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   constexpr int STAGES = Cfg::STAGES;
   static_assert(STAGES >= 2, "pipeline too shallow");
   static_assert(!MMA2 || (CL == 2 && MODE != EPI_STYLE), "the 2-SM MMA needs a CTA pair and the per-warp epilogue");
+  static_assert(!BOX || (CL == 1 && (MODE == EPI_PLAIN || MODE == EPI_AFFINE)), "box tiles: one CTA, PLAIN / AFFINE");
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -626,15 +670,22 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         tma_prefetch_desc(&map_b);
       }
       __syncwarp();
+      // bytes one stage's A box brings (the full box, out-of-bounds fill included)
+      const uint32_t a_bytes = BOX ? (uint32_t)(p.box_tw * p.box_th * p.box_tn) * 128u : (uint32_t)Cfg::A_BYTES;
       int stage = 0;
       uint32_t phase = 0;
       for (int unit = unit0; unit < total_units; unit += unit_step) {
         const int m_tile = (unit / p.num_n_tiles) * CL + crank;
         const int n_tile = unit % p.num_n_tiles;
-        const int m0 = (p.a_mod_tiles > 0 ? m_tile % p.a_mod_tiles : m_tile) * 128;
-        const int w0 = m0 % p.W;
-        const int h0 = (m0 / p.W) % p.H;
-        const int n0 = m0 / (p.W * p.H);
+        int w0, h0, n0;
+        if constexpr (BOX) {
+          box_origin(p, m_tile, w0, h0, n0);
+        } else {
+          const int m0 = (p.a_mod_tiles > 0 ? m_tile % p.a_mod_tiles : m_tile) * 128;
+          w0 = m0 % p.W;
+          h0 = (m0 / p.W) % p.H;
+          n0 = m0 / (p.W * p.H);
+        }
         const int b_row = (m_tile / p.wg_tiles) * p.N_total + n_tile * BLOCK_N;
         for (int tap = 0; tap < p.taps; ++tap) {
           const int dh = tap / p.kw - p.pad;
@@ -650,7 +701,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                                 b_row + crank * (BLOCK_N / 2));
               }
             } else if (elect_one_sync()) {
-              mbar_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
+              mbar_expect_tx(&full_bar[stage], a_bytes + Cfg::B_BYTES);
               tma_load_4d(sa, &map_a, &full_bar[stage], ch * 64, w0 + dw, h0 + dh, n0);
               if (CL == 1)
                 tma_load_2d(sa + Cfg::A_BYTES, &map_b, &full_bar[stage], (tap * p.cin_chunks + ch) * 64, b_row);
@@ -719,18 +770,18 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
       const int n_tile = unit % p.num_n_tiles;
       mbar_wait(&tmem_full[as], aphase);
       tc_fence_after();
-      if constexpr (MODE != EPI_STYLE) {
+      if constexpr (MODE != EPI_STYLE && !BOX) {
         if (p.warp_epi) {
           epilogue_tile_warp<BLOCK_N, MODE>(p, &map_out2, tmem_base, as * BLOCK_N, m_tile * 128, n_tile, &tmem_empty[as],
                                             stg_base, vec, chunk_counter, my_slabs, MMA2);
           continue;
         }
       }
-      epilogue_acc<BLOCK_N, MODE, 2>(p, &map_out, &map_out2, tmem_base, as * BLOCK_N, m_tile * 128, n_tile,
-                                     &tmem_empty[as], stg_base, vec, chunk_counter);
+      epilogue_acc<BLOCK_N, MODE, 2, BOX>(p, &map_out, &map_out2, tmem_base, as * BLOCK_N, m_tile * 128, n_tile,
+                                          &tmem_empty[as], stg_base, vec, chunk_counter);
     }
     // the staging buffers only have to outlive the TMA engine's READS; global visibility comes with grid completion
-    if (MODE != EPI_STYLE && p.warp_epi) {
+    if (MODE != EPI_STYLE && !BOX && p.warp_epi) {
       if (lane == 0) tma_store_wait_read<0>();
     } else if (warp == 2) {
       __syncwarp();
@@ -977,12 +1028,12 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 // ------------------------------------------------------------------------------------------------
 // Host side
 // ------------------------------------------------------------------------------------------------
-template <int BLOCK_N, int MODE, int CL = 1, bool MMA2 = false>
+template <int BLOCK_N, int MODE, int CL = 1, bool MMA2 = false, bool BOX = false>
 static int launch_conv_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo, const CUtensorMap& mo2,
                             const ConvGemmArgs& a, cudaStream_t stream) {
   using Cfg = GemmCfg<BLOCK_N, MODE>;
   static bool configured = false;
-  auto kern = conv_gemm_kernel<BLOCK_N, MODE, CL, MMA2>;
+  auto kern = conv_gemm_kernel<BLOCK_N, MODE, CL, MMA2, BOX>;
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
     if (e != cudaSuccess) {
@@ -1032,6 +1083,18 @@ static int dispatch_block_n(int block_n, const CUtensorMap& ma, const CUtensorMa
     case 64: return launch_conv_gemm<64, MODE>(ma, mb, mo, mo2, a, stream);
     case 128: return launch_conv_gemm<128, MODE>(ma, mb, mo, mo2, a, stream);
     case 256: return launch_conv_gemm<256, MODE>(ma, mb, mo, mo2, a, stream);
+  }
+  set_last_error("bad BLOCK_N %d", block_n);
+  return IRFD_ERR_INVALID_ARGUMENT;
+}
+
+template <int MODE>
+static int dispatch_box(int block_n, const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo,
+                        const ConvGemmArgs& a, cudaStream_t stream) {
+  switch (block_n) {
+    case 64: return launch_conv_gemm<64, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
+    case 128: return launch_conv_gemm<128, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
+    case 256: return launch_conv_gemm<256, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
   }
   set_last_error("bad BLOCK_N %d", block_n);
   return IRFD_ERR_INVALID_ARGUMENT;
@@ -1102,6 +1165,95 @@ extern "C" int irfd_conv_gemm_m_tiles(int n, int h, int w) {
   return (int)((m + 127) / 128);
 }
 
+// Pixel-tile geometry of a conv_gemm launch: the one place the shape rule lives (irfd_conv_gemm_geometry exports it).
+// (H, W, NB) is the 4-D view the A operand's tensor map spans; a pointwise conv is one long row of pixels.
+//   linear: 128 consecutive NHWC pixels form one (tw, th, tn) TMA box (W divides 128 or is a multiple of 128 for 3x3
+//           convs, whole rows / whole images per tile); m tile t = pixels [128 t, 128 t + 128), a ragged last tile.
+//   boxed : every shape the linear geometry rejects (conv_gemm_kernel<..., BOX = true>): a tile is a box of
+//           P = tw*th*tn <= 128 pixels.  W < 128: tw = W, th = min(H, 128 / W), and if th == H, tn = 128 / (H*W)
+//           images (at most NB; with weight groups the largest divisor of the per-group image count, so that every
+//           tile belongs to one group).  W > 128: tw = 128, th = tn = 1, ceil(W / 128) column tiles per row.  Tiles are
+//           ordered image-major, then rows, then columns.
+struct TileGeom {
+  int boxed, tw, th, tn, tiles_w, tiles_h, tiles_n;
+  int H, W, NB;
+};
+
+static int tile_geometry(int n, int h, int w, int ksize, int wgroups, int a_shared, TileGeom* g) {
+  IRFD_CHECK_ARG(ksize == 1 || ksize == 3, "conv_gemm: ksize must be 1 or 3 (got %d)", ksize);
+  IRFD_CHECK_ARG(wgroups >= 1, "conv_gemm: bad weight group count %d", wgroups);
+  const long long m_total_ll = (long long)n * h * w;
+  IRFD_CHECK_ARG(n > 0 && h > 0 && w > 0 && m_total_ll < (1ll << 31) - 256, "conv_gemm: bad pixel count");
+  const int m_total = (int)m_total_ll;
+  int H = h, W = w, NB = n;
+  if (ksize == 1) {  // pointwise conv == plain GEMM over a single long row of pixels
+    H = 1;
+    W = a_shared ? m_total / wgroups : m_total;  // a shared A operand only has one group's rows
+    NB = 1;
+  }
+  g->H = H;
+  g->W = W;
+  g->NB = NB;
+  // linear geometry
+  bool linear = wgroups == 1 || m_total_ll % (128ll * wgroups) == 0;
+  if (W >= 128) {
+    linear = linear && (ksize == 1 || W % 128 == 0);
+    g->tw = 128; g->th = 1; g->tn = 1;
+  } else {
+    const int rows = 128 / W;
+    linear = linear && 128 % W == 0 && (H >= rows ? H % rows == 0 : rows % H == 0);
+    g->tw = W;
+    g->th = H >= rows ? rows : H;
+    g->tn = H >= rows ? 1 : rows / H;
+  }
+  if (linear) {
+    g->boxed = 0;
+    if (W >= 128) {
+      g->tiles_w = (W + 127) / 128;  // pointwise: a ragged last tile
+      g->tiles_h = H;
+      g->tiles_n = NB;
+    } else {
+      g->tiles_w = 1;
+      g->tiles_h = H / g->th;
+      g->tiles_n = (NB + g->tn - 1) / g->tn;
+    }
+    return IRFD_OK;
+  }
+  // box-tiled geometry
+  IRFD_CHECK_ARG(NB % wgroups == 0,
+                 "conv_gemm: %d weight groups need whole tiles per group (n=%d h=%d w=%d ksize=%d)", wgroups, n, h, w,
+                 ksize);
+  g->boxed = 1;
+  if (W > 128) {
+    g->tw = 128; g->th = 1; g->tn = 1;
+  } else {
+    g->tw = W;
+    g->th = H < 128 / W ? H : 128 / W;
+    int tn = 1;
+    if (g->th == H) {
+      tn = 128 / (H * W);
+      if (tn > NB) tn = NB;
+      if (wgroups > 1)
+        while ((NB / wgroups) % tn) --tn;
+    }
+    g->tn = tn;
+  }
+  g->tiles_w = (W + g->tw - 1) / g->tw;
+  g->tiles_h = (H + g->th - 1) / g->th;
+  g->tiles_n = (NB + g->tn - 1) / g->tn;
+  return IRFD_OK;
+}
+
+extern "C" int irfd_conv_gemm_geometry(int n, int h, int w, int ksize, int wgroups, int* out_host) {
+  IRFD_CHECK_ARG(out_host != nullptr, "conv_gemm_geometry: null output");
+  TileGeom g;
+  const int rc = tile_geometry(n, h, w, ksize, wgroups, 0, &g);
+  if (rc != IRFD_OK) return rc;
+  const int v[7] = {g.boxed, g.tw, g.th, g.tn, g.tiles_w, g.tiles_h, g.tiles_n};
+  for (int i = 0; i < 7; ++i) out_host[i] = v[i];
+  return IRFD_OK;
+}
+
 struct BnBwdFold {  // EPI_BNBWD / EPI_BNBWD_RES operands (see ConvGemmArgs)
   const void* z;
   const float *mean, *rstd;
@@ -1125,40 +1277,31 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
   const long long m_total_ll = (long long)n * h * w;
   IRFD_CHECK_ARG(m_total_ll > 0 && m_total_ll < (1ll << 31) - 256, "conv_gemm: bad pixel count");
   const int m_total = (int)m_total_ll;
-  IRFD_CHECK_ARG(wgroups == 1 || (wgroups > 1 && m_total_ll % (128ll * wgroups) == 0),
-                 "conv_gemm: %d weight groups need a whole number of 128-pixel tiles per group (pixels %lld)", wgroups,
-                 m_total_ll);
+  IRFD_CHECK_ARG(wgroups >= 1, "conv_gemm: bad weight group count %d", wgroups);
   IRFD_CHECK_ARG(wgroups == 1 || (mode != EPI_STYLE), "conv_gemm: weight groups are not available in STYLE mode");
   IRFD_CHECK_ARG(!a_shared || (ksize == 1 && wgroups > 1), "conv_gemm: a shared A operand needs ksize 1 and groups > 1");
 
-  // pixel-tile geometry: 128 consecutive NHWC pixels == a (tn, th, tw) box
-  int H = h, W = w, NB = n;
-  if (ksize == 1) {  // pointwise conv == plain GEMM over a single long row of pixels
-    H = 1;
-    W = a_shared ? m_total / wgroups : m_total;  // a shared A operand only has one group's rows
-    NB = 1;
+  TileGeom geo;
+  {
+    const int rc = tile_geometry(n, h, w, ksize, wgroups, a_shared, &geo);
+    if (rc != IRFD_OK) return rc;
   }
-  int tw, th, tn;
-  if (W >= 128) {
-    IRFD_CHECK_ARG(ksize == 1 || W % 128 == 0, "conv_gemm: W=%d must be a multiple of 128", W);
-    tw = 128; th = 1; tn = 1;
-  } else {
-    IRFD_CHECK_ARG(128 % W == 0, "conv_gemm: W=%d must divide 128", W);
-    tw = W;
-    const int rows = 128 / W;
-    if (H >= rows) {
-      IRFD_CHECK_ARG(H % rows == 0, "conv_gemm: H=%d must be a multiple of %d", H, rows);
-      th = rows; tn = 1;
-    } else {
-      IRFD_CHECK_ARG(rows % H == 0, "conv_gemm: H=%d must divide %d", H, rows);
-      th = H; tn = rows / H;
-    }
-  }
+  const bool boxed = geo.boxed != 0;
+  IRFD_CHECK_ARG(!boxed || mode == EPI_PLAIN || mode == EPI_AFFINE,
+                 "conv_gemm: n=%d h=%d w=%d (ksize %d) needs box tiles, which serve the plain and affine epilogues only "
+                 "(mode %d)", n, h, w, ksize, mode);
+  const int H = geo.H, W = geo.W, NB = geo.NB;
+  const int tw = geo.tw, th = geo.th, tn = geo.tn;
 
   ConvGemmArgs a;
   a.M_total = m_total;
   a.N_total = cout;
-  a.num_m_tiles = (m_total + 127) / 128;
+  a.num_m_tiles = boxed ? geo.tiles_w * geo.tiles_h * geo.tiles_n : (m_total + 127) / 128;
+  a.box_tw = tw;
+  a.box_th = th;
+  a.box_tn = tn;
+  a.box_tiles_w = geo.tiles_w;
+  a.box_tiles_h = geo.tiles_h;
   a.taps = ksize * ksize;
   a.kw = ksize;
   a.pad = ksize / 2;
@@ -1177,7 +1320,7 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     IRFD_CHECK_ARG(h * w >= 64, "conv_gemm: STYLE mode needs >= 64 pixels per image");
   }
   if (mode == EPI_STATS) IRFD_CHECK_ARG(stat_sum && stat_sq, "conv_gemm: STATS mode needs stat buffers");
-  a.warp_epi = (mode != EPI_STYLE && m_total % 128 == 0 && warp_epi_mode() != 0) ? 1 : 0;
+  a.warp_epi = (mode != EPI_STYLE && !boxed && m_total % 128 == 0 && warp_epi_mode() != 0) ? 1 : 0;
   a.bn_z = nullptr;
   a.bn_mean = a.bn_rstd = nullptr;
   for (int i = 0; i < 4; ++i) a.bn_gamma[i] = a.bn_beta[i] = nullptr;
@@ -1225,14 +1368,14 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
                  "conv_gemm: BLOCK_N %d incompatible with Cout %d", block_n, cout);
   // halo-reuse kernel: 3x3, rows of >= 128 pixels, Cout of one 64/128-wide tile (the fabric-bound generator layers)
   const int hmode = halo_mode();
-  const bool use_halo = hmode != 0 && mode != EPI_BNBWD && mode != EPI_BNBWD_RES && wgroups == 1 && ksize == 3 && W % 128 == 0 && H % 2 == 0 &&
+  const bool use_halo = hmode != 0 && !boxed && mode != EPI_BNBWD && mode != EPI_BNBWD_RES && wgroups == 1 && ksize == 3 && W % 128 == 0 && H % 2 == 0 &&
                         (cout == 64 || cout == 128) &&
                         (force_block_n == 0 || force_block_n == cout);
   if (use_halo) block_n = cout;
   a.num_n_tiles = cout / block_n;
   // CTA pairs (multicast weight tiles): two consecutive m tiles must belong to the same weight group / A matrix
   int cluster = 1;
-  if (!use_halo && (cluster_mode() != 0 || mma2_mode() != 0) && block_n >= 128 && a.num_m_tiles % 2 == 0 &&
+  if (!use_halo && !boxed && (cluster_mode() != 0 || mma2_mode() != 0) && block_n >= 128 && a.num_m_tiles % 2 == 0 &&
       (wgroups == 1 || a.wg_tiles % 2 == 0) && (a.a_mod_tiles == 0 || a.a_mod_tiles % 2 == 0))
     cluster = (mma2_mode() != 0 && a.warp_epi && (mode == EPI_PLAIN || mode == EPI_STATS || mode == EPI_BNBWD)) ? 3 : 2;
 
@@ -1256,6 +1399,15 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     const uint32_t box[2] = {64, (uint32_t)(block_n / (cluster > 1 ? 2 : 1))};  // a CTA pair loads half a weight tile each
     int rc = make_tmap_bf16(&mb, wk, 2, dims, str, box, true);
     if (rc) return rc;
+  }
+  if (boxed) {  // the epilogue stores each tile as one 4-D box over [NB][H][W][cout]; TMA clips what lies outside
+    const uint64_t dims[4] = {(uint64_t)cout, (uint64_t)W, (uint64_t)H, (uint64_t)NB};
+    const uint64_t str[3] = {(uint64_t)cout * 2, (uint64_t)W * cout * 2, (uint64_t)H * W * cout * 2};
+    const uint32_t box[4] = {64, (uint32_t)tw, (uint32_t)th, (uint32_t)tn};
+    const int rc = make_tmap_bf16(&mo, out, 4, dims, str, box, true);
+    if (rc) return rc;
+    if (mode == EPI_PLAIN) return dispatch_box<EPI_PLAIN>(block_n, ma, mb, mo, a, stream);
+    return dispatch_box<EPI_AFFINE>(block_n, ma, mb, mo, a, stream);
   }
   {
     const uint64_t dims[2] = {(uint64_t)cout, (uint64_t)m_total};

@@ -47,9 +47,9 @@ constexpr int kStemPixPar = 8;  // output pixels in flight per block pass
 __global__ void __launch_bounds__(256)
 im2col_stem_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col, int N, int H, int W, int kpad) {
   extern __shared__ float srow[];  // [3][7][W + 6]
-  const int Ho = H / 2, Wo = W / 2, P = W + 6;
+  const int Ho = (H + 1) / 2, Wo = (W + 1) / 2, P = W + 6;
   const int n = blockIdx.x / Ho, oh = blockIdx.x - n * Ho;
-  // stage: one warp per (channel, kernel row) input row, 16-byte loads (W % 4 == 0, host-checked), all of a warp's loads
+  // stage: one warp per (channel, kernel row) input row, 16-byte loads when W % 4 == 0 (scalar otherwise), all of a warp's loads
   // independent (the per-element version walked 29 dependent iterations with two divisions each)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   for (int cr = warp; cr < 21; cr += nwarps) {  // cr = c * 7 + kh
@@ -60,7 +60,7 @@ im2col_stem_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col,
       dst[lane] = 0.f;
       dst[P - 3 + lane] = 0.f;
     }
-    if (ih >= 0 && ih < H) {
+    if (ih >= 0 && ih < H && (W & 3) == 0) {
       const float4* src = reinterpret_cast<const float4*>(x + (((size_t)n * 3 + c) * H + ih) * W);
       for (int j = lane; j < W / 4; j += 32) {
         const float4 q = __ldg(src + j);
@@ -69,6 +69,9 @@ im2col_stem_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col,
         dst[5 + 4 * j] = q.z;
         dst[6 + 4 * j] = q.w;
       }
+    } else if (ih >= 0 && ih < H) {  // W % 4 != 0: rows are not 16-byte aligned, scalar loads
+      const float* src = x + (((size_t)n * 3 + c) * H + ih) * W;
+      for (int j = lane; j < W; j += 32) dst[3 + j] = __ldg(src + j);
     } else {
       for (int j = lane; j < W; j += 32) dst[3 + j] = 0.f;
     }
@@ -94,7 +97,7 @@ im2col_stem_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col,
 // 3x3 stride-2 pad-1 im2col on NHWC bf16: col[pix][tap*C + c]
 __global__ void im2col_3x3s2_kernel(const __nv_bfloat16* __restrict__ a, __nv_bfloat16* __restrict__ col, int N, int H,
                                     int W, int C) {
-  const unsigned Ho = H / 2, Wo = W / 2, vc = C / 8;
+  const unsigned Ho = (H + 1) / 2, Wo = (W + 1) / 2, vc = C / 8;
   const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;  // host checks total < 2^32
   const size_t total = (size_t)N * Ho * Wo * 9 * vc;
   if (idx >= total) return;
@@ -145,7 +148,7 @@ __global__ void col2im_3x3s2_kernel(const __nv_bfloat16* __restrict__ dcol, __nv
 // 1x1 stride-2 gather: out[n,oh,ow,:] = a[n,2oh,2ow,:]
 __global__ void subsample2_kernel(const __nv_bfloat16* __restrict__ a, __nv_bfloat16* __restrict__ out, int N, int H,
                                   int W, int C) {
-  const unsigned Ho = H / 2, Wo = W / 2, vc = C / 8;
+  const unsigned Ho = (H + 1) / 2, Wo = (W + 1) / 2, vc = C / 8;
   const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;  // host checks total < 2^32
   if (idx >= (size_t)N * Ho * Wo * vc) return;
   const int v = idx % vc;
@@ -184,7 +187,7 @@ __global__ void scatter_add_s2_kernel(const __nv_bfloat16* __restrict__ a, const
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void maxpool_fwd_kernel(const __nv_bfloat16* __restrict__ a, __nv_bfloat16* __restrict__ out,
                                    uint8_t* __restrict__ arg, int N, int H, int W, int C) {
-  const unsigned Ho = H / 2, Wo = W / 2, vc = C / 8;
+  const unsigned Ho = (H + 1) / 2, Wo = (W + 1) / 2, vc = C / 8;
   const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;  // host checks total < 2^32
   if (idx >= (size_t)N * Ho * Wo * vc) return;
   const int v = idx % vc;
@@ -375,19 +378,19 @@ extern "C" int irfd_pack_conv_weight(const float* w, void* dst, int o, int i, in
 }
 
 extern "C" int irfd_im2col_stem(const float* x, void* col, int n, int h, int w, int kpad, cudaStream_t stream) {
-  IRFD_CHECK_ARG(x && col && kpad >= 152 && kpad % 8 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_stem: bad argument");
+  IRFD_CHECK_ARG(x && col && kpad >= 152 && kpad % 8 == 0 && h > 0 && w > 0, "im2col_stem: bad argument");
   const size_t smem = (size_t)21 * (w + 6) * sizeof(float);
-  IRFD_CHECK_ARG(n > 0 && smem <= 48 * 1024, "im2col_stem: image too wide for the row stage (W <= 579)");
-  IRFD_CHECK_ARG(kStemPixPar * (kpad / 8) <= 256 && (kpad / 8) % 4 == 0 && w % 4 == 0,
-                 "im2col_stem: kpad a multiple of 32 and <= 256, W a multiple of 4");
-  im2col_stem_kernel<<<(unsigned)(n * (h / 2)), kStemPixPar * (kpad / 8), smem, stream>>>(x, BF(col), n, h, w, kpad);
+  IRFD_CHECK_ARG(n > 0 && smem <= 48 * 1024, "im2col_stem: image too wide for the row stage (W <= 579, got %d)", w);
+  IRFD_CHECK_ARG(kStemPixPar * (kpad / 8) <= 256 && (kpad / 8) % 4 == 0, "im2col_stem: kpad a multiple of 32 and <= 256");
+  im2col_stem_kernel<<<(unsigned)(n * ((h + 1) / 2)), kStemPixPar * (kpad / 8), smem, stream>>>(x, BF(col), n, h, w,
+                                                                                              kpad);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
 }
 
 extern "C" int irfd_im2col_3x3s2(const void* a, void* col, int n, int h, int w, int c, cudaStream_t stream) {
-  IRFD_CHECK_ARG(a && col && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_3x3s2: bad argument");
-  const size_t total = (size_t)n * (h / 2) * (w / 2) * 9 * (c / 8);
+  IRFD_CHECK_ARG(a && col && c % 8 == 0 && h > 0 && w > 0, "im2col_3x3s2: bad argument");
+  const size_t total = (size_t)n * ((h + 1) / 2) * ((w + 1) / 2) * 9 * (c / 8);
   CHECK_TOTAL32(total);
   im2col_3x3s2_kernel<<<GRID1D(total)>>>(CBF(a), BF(col), n, h, w, c);
   IRFD_CHECK_LAUNCH();
@@ -404,8 +407,8 @@ extern "C" int irfd_col2im_3x3s2(const void* dcol, void* dx, int n, int h, int w
 }
 
 extern "C" int irfd_subsample2(const void* a, void* out, int n, int h, int w, int c, cudaStream_t stream) {
-  IRFD_CHECK_ARG(a && out && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "subsample2: bad argument");
-  const size_t total = (size_t)n * (h / 2) * (w / 2) * (c / 8);
+  IRFD_CHECK_ARG(a && out && c % 8 == 0 && h > 0 && w > 0, "subsample2: bad argument");
+  const size_t total = (size_t)n * ((h + 1) / 2) * ((w + 1) / 2) * (c / 8);
   CHECK_TOTAL32(total);
   subsample2_kernel<<<GRID1D(total)>>>(CBF(a), BF(out), n, h, w, c);
   IRFD_CHECK_LAUNCH();
@@ -424,8 +427,8 @@ extern "C" int irfd_scatter_add_s2(const void* a, const void* b, void* out, int 
 
 extern "C" int irfd_maxpool_fwd(const void* a, void* out, void* argmax, int n, int h, int w, int c,
                                 cudaStream_t stream) {
-  IRFD_CHECK_ARG(a && out && argmax && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "maxpool_fwd: bad argument");
-  const size_t total = (size_t)n * (h / 2) * (w / 2) * (c / 8);
+  IRFD_CHECK_ARG(a && out && argmax && c % 8 == 0 && h > 0 && w > 0, "maxpool_fwd: bad argument");
+  const size_t total = (size_t)n * ((h + 1) / 2) * ((w + 1) / 2) * (c / 8);
   CHECK_TOTAL32(total);
   maxpool_fwd_kernel<<<GRID1D(total)>>>(CBF(a), BF(out), reinterpret_cast<uint8_t*>(argmax), n, h, w, c);
   IRFD_CHECK_LAUNCH();

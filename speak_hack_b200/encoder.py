@@ -18,6 +18,31 @@ from . import ops
 
 BN_EPS = 1e-5
 BN_MOMENTUM = 0.1
+# widest image the stem's im2col stages (21 input rows of W + 6 fp32 in 48 KB of shared memory)
+MAX_STEM_W = 579
+MIN_HW = 32
+
+
+def check_inference_shape(x) -> None:
+    """The eval-mode, no-autograd pass runs at any 32 <= H, W with W <= 579 (box-tiled convs where 128 consecutive
+    pixels are not one tile, ceil-sized stride-2 layers like torchvision)."""
+    h, w = x.shape[2], x.shape[3]
+    if h < MIN_HW or w < MIN_HW or w > MAX_STEM_W:
+        raise ops._lib.IrfdError(f"ResNet50Encoder: eval-mode inference needs {MIN_HW} <= H, W and W <= {MAX_STEM_W}, "
+                                 f"got {tuple(x.shape)}")
+
+
+def trainable_shape(n: int, h: int, w: int) -> bool:
+    """Train-mode and differentiated passes (batch statistics in the conv epilogues, the backward kernels) need H and W
+    multiples of 32 and every conv of the n-image batch on the linear pixel-tile geometry (ops.conv_geometry)."""
+    if h % 32 or w % 32 or w > MAX_STEM_W:
+        return False
+    for i, (hs, ws) in enumerate(ops.resnet_stage_hw(h, w)):
+        for k in ((1, 3) if i > 0 else (1,)):  # 3x3 stride-1 convs from layer1 on; 1x1 GEMMs at every stage
+            g = ops.conv_geometry(n, hs, ws, k)
+            if g is None or g[0]:
+                return False
+    return True
 
 
 class Bottleneck(nn.Module):
@@ -87,7 +112,7 @@ def _encoder_inference(enc, x, col0=None):
     m0 = col0.shape[0]
     sc, sh = ops.bn_eval_affine(enc[1])
     a0 = ops.conv_gemm_affine(col0.view(1, 1, m0, 192), ops.pack_conv_weight(enc[0].weight, ops.PACK_FLAT, kpad=192), 1,
-                              sc, sh, relu=True).view(n, h // 2, w // 2, 64)
+                              sc, sh, relu=True).view(n, ops.half_up(h), ops.half_up(w), 64)
     cur, _ = ops.maxpool_fwd(a0)
     for li in range(4, 8):
         for blk in enc[li]:
@@ -102,7 +127,7 @@ def _encoder_inference(enc, x, col0=None):
             else:
                 col2 = ops.im2col_3x3s2(a1)
                 a2 = ops.conv_gemm_affine(col2.view(1, 1, col2.shape[0], 9 * planes), wk2, 1, sc, sh,
-                                          relu=True).view(nb, hh // 2, ww // 2, planes)
+                                          relu=True).view(nb, ops.half_up(hh), ops.half_up(ww), planes)
             if blk.downsample is not None:
                 xs = ops.subsample2(cur) if blk.stride == 2 else cur
                 sc, sh = ops.bn_eval_affine(blk.downsample[1])
@@ -294,15 +319,22 @@ class ResNet50Encoder(nn.Sequential):
     def forward(self, x):
         if not x.is_cuda:
             raise ops._lib.IrfdError("ResNet50Encoder: CUDA tensors only (no CPU fallback on the IRFD hot path)")
-        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] % 32 or x.shape[3] % 32:
-            raise ops._lib.IrfdError(f"ResNet50Encoder: expected [N,3,H,W] with H,W multiples of 32, got {tuple(x.shape)}")
+        if x.dim() != 4 or x.shape[1] != 3:
+            raise ops._lib.IrfdError(f"ResNet50Encoder: expected [N,3,H,W], got {tuple(x.shape)}")
         return self._run(x, 1, None)
 
     def _run(self, x, groups, stem_cols):
         params = self._flat_params()
         recorded = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
         if not self.training and not recorded:
+            check_inference_shape(x)
             return _encoder_inference(self, x, stem_cols)  # inference: BN/ReLU/residual folded into the convs
+        # refused before any launch, so the BatchNorm running buffers and counters stay untouched
+        if not trainable_shape(x.size(0), x.shape[2], x.shape[3]):
+            mode = "train-mode" if self.training else "differentiated eval-mode"
+            raise ops._lib.IrfdError(f"ResNet50Encoder: a {mode} pass needs H, W multiples of 32 (W <= {MAX_STEM_W}) and "
+                                     f"128-pixel tiles of whole rows / images at every stage, got {tuple(x.shape)}; "
+                                     "eval-mode inference under no_grad runs at any 32 <= H, W")
         return _EncoderFn.apply(x, self, groups, stem_cols, recorded, *params)
 
     def can_group(self, x: torch.Tensor, groups: int) -> bool:

@@ -35,7 +35,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
-from .encoder import BN_EPS, BN_MOMENTUM, ResNet50Encoder
+from .encoder import BN_EPS, BN_MOMENTUM, MAX_STEM_W, MIN_HW, ResNet50Encoder, trainable_shape
 
 
 # IRFD_BN_FOLD (default 1): the reduce pass of bn1 / bn2's backward runs in the epilogue of the dgrad GEMM that produces
@@ -71,7 +71,7 @@ def _group_inference(grp: "EncoderGroup", x, col0=None):
         col0 = ops.im2col_stem(x, 192)
     sc, sh = ops.bn_eval_affine_sets([e[1] for e in encs])
     a0 = ops.conv_gemm_affine_grouped(col0, _stack_pack([e[0] for e in encs], ops.PACK_FLAT, 192), 1, sc, sh, relu=True,
-                                      wgroups=E, a_shared=True).view(E * n, h // 2, w // 2, 64)
+                                      wgroups=E, a_shared=True).view(E * n, ops.half_up(h), ops.half_up(w), 64)
     cur, _ = ops.maxpool_fwd(a0)
     for li in range(4, 8):
         for bi in range(len(encs[0][li])):
@@ -88,7 +88,7 @@ def _group_inference(grp: "EncoderGroup", x, col0=None):
             else:
                 col2 = ops.im2col_3x3s2(a1)
                 a2 = ops.conv_gemm_affine_grouped(col2.view(1, 1, col2.shape[0], 9 * planes), wk2, 1, sc, sh, relu=True,
-                                                  wgroups=E).view(nb, hh // 2, ww // 2, planes)
+                                                  wgroups=E).view(nb, ops.half_up(hh), ops.half_up(ww), planes)
             if blks[0].downsample is not None:
                 xs = ops.subsample2(cur) if blks[0].stride == 2 else cur
                 sc, sh = ops.bn_eval_affine_sets([b.downsample[1] for b in blks])
@@ -341,10 +341,25 @@ class EncoderGroup:
         encs = self.encoders
         if not (x.is_cuda and x.dim() == 4 and x.shape[1] == 3 and x.size(0) % groups == 0):
             return False
-        if x.shape[2] % 32 or x.shape[3] % 32 or len({e.training for e in encs}) != 1:
+        if len({e.training for e in encs}) != 1:
+            return False
+        h, w = x.shape[2], x.shape[3]
+        if not encs[0].training:
+            # eval mode: every grouped launch must give each encoder whole tiles of its x.size(0) images (ONE statistic
+            # group, the running statistics): the flat GEMMs (stem, 1x1, stride-2 im2col) need a multiple of 128 pixels
+            # per encoder, the 3x3 convs a tile geometry with whole images per encoder
+            if h < MIN_HW or w < MIN_HW or w > MAX_STEM_W:
+                return False
+            E, n = len(encs), x.size(0)
+            for i, (hs, ws) in enumerate(ops.resnet_stage_hw(h, w)):
+                for k in ((1, 3) if i > 0 else (1,)):
+                    if ops.conv_geometry(E * n, hs, ws, k, E) is None:
+                        return False
+            return True
+        if h % 32 or w % 32 or not trainable_shape(x.size(0), h, w):
             return False
         per_group = x.size(0) // groups
-        return (per_group * (x.shape[2] // 32) * (x.shape[3] // 32)) % 128 == 0
+        return (per_group * (h // 32) * (w // 32)) % 128 == 0
 
     def __call__(self, x: torch.Tensor, groups: int = 1, stem_cols=None):
         """Returns features [E, N, 2048, 1, 1]: out[e] == encoders[e].forward_groups(x, groups)."""

@@ -15,7 +15,7 @@ import torch.nn as nn
 
 from . import ops
 from .discriminator import StyleDiscriminator
-from .encoder import ResNet50Encoder
+from .encoder import ResNet50Encoder, _encoder_inference, check_inference_shape
 from .encoder_group import EncoderGroup
 from .generator import StyleGenerator
 
@@ -261,7 +261,21 @@ def _irfd_forward_static_stacked(self: IRFD, x, ctrl):
     grp = self.encoder_group
     b = x.size(0) // 2
     diff = torch.is_grad_enabled() and x.requires_grad
-    if not grp.can_run(x, 2) or (diff and not grp.encoders[0].training):
+    training = grp.encoders[0].training
+    if not training and not diff and not grp.can_run(x, 2):
+        # eval-mode inference at a size the lockstep pass cannot tile: the three encoders one after the other on the
+        # stacked batch (same arithmetic per pixel, so the same features), sharing the stem's im2col matrix
+        encs = grp.encoders
+        if not (x.is_cuda and x.dim() == 4 and x.shape[1] == 3) or len({e.training for e in encs}) != 1:
+            raise ops._lib.IrfdError(f"IRFD.forward_static: bad batch {tuple(x.shape)} / encoder modes")
+        check_inference_shape(x)
+        with torch.no_grad():
+            xf = x.contiguous().to(torch.float32)
+            col0 = ops.im2col_stem(xf, 192)
+            f = torch.stack([_encoder_inference(e, xf, col0) for e in encs])
+        gen = _SwapCatStackedFn.apply(ctrl, f)
+        return self.Gd.forward_static(gen, ctrl, 1, b_first=b), f, b
+    if not grp.can_run(x, 2) or (diff and not training):
         raise ops._lib.IrfdError(f"IRFD.forward_static: batch {tuple(x.shape)} cannot run as one lockstep encoder pass "
                                  "(needs pairs x (H/32) x (W/32) to be a multiple of 128); use IRFD.forward")
     if diff:

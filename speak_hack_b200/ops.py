@@ -681,22 +681,45 @@ def bn_backward_finish_sets(g, z, mean, rstd, gammas, partial, dgammas=None, dbe
     return dz, dgammas, dbetas
 
 
+def conv_geometry(n: int, h: int, w: int, ksize: int, wgroups: int = 1):
+    """Pixel-tile geometry the conv GEMM uses for this shape (irfd_conv_gemm_geometry, host-only, no CUDA call):
+    (boxed, tw, th, tn, tiles_w, tiles_h, tiles_n), or None when no geometry serves the shape."""
+    out = (ctypes.c_int * 7)()
+    if _lib.load().irfd_conv_gemm_geometry(n, h, w, ksize, wgroups, out) != _lib.IRFD_OK:
+        return None
+    return tuple(out)
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 # layout / pooling
 # ----------------------------------------------------------------------------------------------------------------------
+def half_up(x: int) -> int:
+    """Output size of every stride-2 layer of ResNet-50 (7x7/2 p3, MaxPool 3/2 p1, 3x3/2 p1, 1x1/2): ceil(x / 2)."""
+    return (x + 1) // 2
+
+
+def resnet_stage_hw(h: int, w: int):
+    """Feature-map sizes of a ResNet-50 on an h x w image: [stem conv, layer1 (after the maxpool), layer2, layer3,
+    layer4], each (H, W) — torchvision's arithmetic for any size."""
+    sizes = [(half_up(h), half_up(w))]
+    for _ in range(4):  # the maxpool (layer1 keeps its size), then the stride-2 first blocks of layer2..4
+        sizes.append((half_up(sizes[-1][0]), half_up(sizes[-1][1])))
+    return sizes
+
+
 def im2col_stem(x: torch.Tensor, kpad: int = 192) -> torch.Tensor:
     _chk(x, F32, "x")
     n, c, h, w = x.shape
     if c != 3:
         raise _lib.IrfdError("im2col_stem expects 3 input channels")
-    col = torch.empty((n * (h // 2) * (w // 2), kpad), dtype=BF16, device=x.device)
+    col = torch.empty((n * half_up(h) * half_up(w), kpad), dtype=BF16, device=x.device)
     _call("irfd_im2col_stem", x.data_ptr(), col.data_ptr(), n, h, w, kpad, _stream())
     return col
 
 
 def im2col_3x3s2(a: torch.Tensor) -> torch.Tensor:
     n, h, w, c = a.shape
-    col = torch.empty((n * (h // 2) * (w // 2), 9 * c), dtype=BF16, device=a.device)
+    col = torch.empty((n * half_up(h) * half_up(w), 9 * c), dtype=BF16, device=a.device)
     _call("irfd_im2col_3x3s2", a.data_ptr(), col.data_ptr(), n, h, w, c, _stream())
     return col
 
@@ -709,7 +732,7 @@ def col2im_3x3s2(dcol: torch.Tensor, n, h, w, c) -> torch.Tensor:
 
 def subsample2(a: torch.Tensor) -> torch.Tensor:
     n, h, w, c = a.shape
-    out = torch.empty((n, h // 2, w // 2, c), dtype=BF16, device=a.device)
+    out = torch.empty((n, half_up(h), half_up(w), c), dtype=BF16, device=a.device)
     _call("irfd_subsample2", a.data_ptr(), out.data_ptr(), n, h, w, c, _stream())
     return out
 
@@ -723,8 +746,8 @@ def scatter_add_s2(a: Optional[torch.Tensor], b: torch.Tensor) -> torch.Tensor:
 
 def maxpool_fwd(a: torch.Tensor):
     n, h, w, c = a.shape
-    out = torch.empty((n, h // 2, w // 2, c), dtype=BF16, device=a.device)
-    arg = torch.empty((n, h // 2, w // 2, c), dtype=torch.uint8, device=a.device)
+    out = torch.empty((n, half_up(h), half_up(w), c), dtype=BF16, device=a.device)
+    arg = torch.empty((n, half_up(h), half_up(w), c), dtype=torch.uint8, device=a.device)
     _call("irfd_maxpool_fwd", a.data_ptr(), out.data_ptr(), arg.data_ptr(), n, h, w, c, _stream())
     return out, arg
 
