@@ -21,10 +21,14 @@ of the tensor peak, 18-55 us launches against 6-26 us bounds).  `EncoderGroup` r
   activation gradient is written once, already masked, and read once; the block outputs keep their ReLU mask as a bit
   plane (`irfd_bn_apply_sets(mask_bits)`) that bn3's backward reads instead of the activation.
 
-Numerically the forward of the grouped pass is the per-encoder pass: same kernels, same tiles, same summation order
-per tile (tests/test_gpu_encoder_group.py: features and BN buffers bit-identical).  The backward sums the BatchNorm
-statistics of bn1 / bn2 per 128-pixel tile instead of per row block: same terms in a different fp32 order
-(IRFD_BN_FOLD=0 restores the per-encoder launches and gradients equal to 3e-6).
+This module is the only implementation of the encoder forward, backward and inference: a lone encoder call
+(`ResNet50Encoder.forward` / `forward_groups`) runs as the one-member group `EncoderGroup([enc])`.
+
+Numerically the forward of an E-encoder pass is E one-encoder passes: same kernels, same tiles, same summation order
+per tile (tests/test_gpu_encoder_group.py: features and BN buffers bit-identical).  With E > 1 the backward sums the
+BatchNorm statistics of bn1 / bn2 per 128-pixel tile instead of per row block: same terms in a different fp32 order
+(IRFD_BN_FOLD=0 restores the separate launches and gradients equal to 3e-6).  A lone encoder never folds, so its
+gradients do not depend on the setting.
 """
 from __future__ import annotations
 
@@ -105,24 +109,35 @@ def _group_inference(grp: "EncoderGroup", x, col0=None):
 class _EncoderGroupFn(torch.autograd.Function):
     """forward(x [N,3,H,W] fp32, group, stat_groups, col0, recorded, *params) -> features [E, N, 2048, 1, 1] fp32.
 
-    Train mode only (eval-mode forwards without autograd go through _group_inference; eval-mode forwards WITH autograd
-    through the per-encoder path).  params = the encoders' parameters, encoder after encoder, in _flat_params() order.
-    x stacks `stat_groups` independent batches along dim 0 (IRFD: source and target images): BatchNorm statistics are
-    per (encoder, group) and each encoder's running buffers are updated group by group, like separate calls."""
+    Train mode, and eval mode with autograd (E == 1 only); eval-mode forwards without autograd go through
+    _group_inference.  params = the encoders' parameters, encoder after encoder, in _flat_params() order.
+    In train mode x stacks `stat_groups` independent batches along dim 0 (IRFD: source and target images): BatchNorm
+    statistics are per (encoder, group) and each encoder's running buffers are updated group by group, like separate
+    calls.  In eval mode every BatchNorm normalises with its running statistics and no buffer changes."""
 
     @staticmethod
     def forward(ctx, x, grp, stat_groups, col0, recorded, *params):
         encs: List[ResNet50Encoder] = grp.encoders
         E = len(encs)
-        G = stat_groups
+        train = encs[0].training
+        assert train or E == 1
+        G = stat_groups if train else 1  # eval mode: the shared running statistics, no groups needed
         GT = E * G  # statistic groups of a stacked tensor: encoder-major, then the caller's groups
         # reentrant-checkpoint semantics of the reference (model.py:84-90, SURVEY Q3): a differentiated pass updates the
         # BN running buffers twice, forward order then reverse order
-        U = 2 if (recorded and all(getattr(e, "_recompute_bn_update", False) for e in encs)) else 1
+        U = 2 if (train and recorded and all(getattr(e, "_recompute_bn_update", False) for e in encs)) else 1
         x = x.contiguous().to(torch.float32)
         n, _, h, w = x.shape
 
+        def conv(xx, wk, ksize, **kw):
+            """Forward conv; in train mode its epilogue also gathers the BatchNorm statistics."""
+            if train:
+                return ops.conv_gemm_grouped(xx, wk, ksize, ops.EPI_STATS, wgroups=E, **kw)
+            return ops.conv_gemm_grouped(xx, wk, ksize, wgroups=E, **kw), None, None
+
         def stats(bns, s, q, rows_total):
+            if not train:
+                return _Stats(bns[0].running_mean, ops.bn_eval_rstd(bns[0].running_var, BN_EPS))
             mean, rstd = ops.bn_finalize_sets(s, q, rows_total // GT, BN_EPS, BN_MOMENTUM,
                                               [b.running_mean for b in bns], [b.running_var for b in bns], U, G, E)
             return _Stats(mean, rstd)
@@ -135,8 +150,7 @@ class _EncoderGroupFn(torch.autograd.Function):
         if col0 is None:
             col0 = ops.im2col_stem(x, 192)
         bn0 = [e[1] for e in encs]
-        z0, s, q = ops.conv_gemm_grouped(col0, _stack_pack([e[0] for e in encs], ops.PACK_FLAT, 192), 1, ops.EPI_STATS,
-                                         wgroups=E, a_shared=True)
+        z0, s, q = conv(col0, _stack_pack([e[0] for e in encs], ops.PACK_FLAT, 192), 1, a_shared=True)
         h1, w1 = h // 2, w // 2
         z0 = z0.view(E * n, h1, w1, 64)
         st0 = stats(bn0, s, q, E * n * h1 * w1)
@@ -149,8 +163,7 @@ class _EncoderGroupFn(torch.autograd.Function):
                 blks = [e[li][bi] for e in encs]
                 xin = cur
                 nb, hh, ww, _cin = xin.shape
-                z1, s, q = ops.conv_gemm_grouped(xin, _stack_pack([b.conv1 for b in blks], ops.PACK_FPROP), 1,
-                                                 ops.EPI_STATS, wgroups=E)
+                z1, s, q = conv(xin, _stack_pack([b.conv1 for b in blks], ops.PACK_FPROP), 1)
                 bn1 = [b.bn1 for b in blks]
                 st1 = stats(bn1, s, q, nb * hh * ww)
                 a1 = apply(z1, st1, bn1)
@@ -158,26 +171,23 @@ class _EncoderGroupFn(torch.autograd.Function):
                 wk2 = _stack_pack([b.conv2 for b in blks], ops.PACK_FPROP)
                 col2 = None
                 if blks[0].stride == 1:
-                    z2, s, q = ops.conv_gemm_grouped(a1, wk2, 3, ops.EPI_STATS, wgroups=E)
+                    z2, s, q = conv(a1, wk2, 3)
                     ho, wo = hh, ww
                 else:
                     col2 = ops.im2col_3x3s2(a1)
                     ho, wo = hh // 2, ww // 2
-                    z2, s, q = ops.conv_gemm_grouped(col2.view(1, 1, col2.shape[0], 9 * planes), wk2, 1, ops.EPI_STATS,
-                                                     wgroups=E)
+                    z2, s, q = conv(col2.view(1, 1, col2.shape[0], 9 * planes), wk2, 1)
                     z2 = z2.view(nb, ho, wo, planes)
                 bn2 = [b.bn2 for b in blks]
                 st2 = stats(bn2, s, q, nb * ho * wo)
                 a2 = apply(z2, st2, bn2)
-                z3, s, q = ops.conv_gemm_grouped(a2, _stack_pack([b.conv3 for b in blks], ops.PACK_FPROP), 1,
-                                                 ops.EPI_STATS, wgroups=E)
+                z3, s, q = conv(a2, _stack_pack([b.conv3 for b in blks], ops.PACK_FPROP), 1)
                 bn3 = [b.bn3 for b in blks]
                 st3 = stats(bn3, s, q, nb * ho * wo)
                 xs = zd = std = None
                 if blks[0].downsample is not None:
                     xs = ops.subsample2(xin) if blks[0].stride == 2 else xin
-                    zd, s, q = ops.conv_gemm_grouped(xs, _stack_pack([b.downsample[0] for b in blks], ops.PACK_FPROP), 1,
-                                                     ops.EPI_STATS, wgroups=E)
+                    zd, s, q = conv(xs, _stack_pack([b.downsample[0] for b in blks], ops.PACK_FPROP), 1)
                     dbn = [b.downsample[1] for b in blks]
                     std = stats(dbn, s, q, nb * ho * wo)
                     out = apply(z3, st3, bn3, res=zd, want_mask=recorded,
@@ -190,18 +200,22 @@ class _EncoderGroupFn(torch.autograd.Function):
                 S["blocks"].append((li, blks, xin, z1, st1, a1, col2, z2, st2, a2, z3, st3, xs, zd, std, obits))
                 cur = out
         feat = ops.avgpool_fwd(cur)
-        counters = [c for e in encs for c in e._bn_counters()]
-        torch._foreach_add_(counters, G * U)  # nn.BatchNorm2d bookkeeping (one fused increment)
+        if train:  # nn.BatchNorm2d bookkeeping (one fused increment)
+            torch._foreach_add_([c for e in encs for c in e._bn_counters()], G * U)
         S["final_hw"] = (cur.shape[1], cur.shape[2])
-        ctx.grp, ctx.S, ctx.G = grp, S, G
+        ctx.grp, ctx.S, ctx.G, ctx.train = grp, S, G, train
         return feat.view(E, n, -1, 1, 1)
 
     @staticmethod
     def backward(ctx, dfeat):
-        grp, S, G = ctx.grp, ctx.S, ctx.G
+        grp, S, G, train = ctx.grp, ctx.S, ctx.G, ctx.train
         encs = grp.encoders
         E = len(encs)
         GT = E * G
+        # the folded reduce passes sum in another fp32 order, which the train-mode stack amplifies
+        # (scripts/fold_probe.py): a lone encoder keeps the separate launches, so its gradients do not depend on the
+        # setting
+        fold, fold3 = fold_bn_reduce and E > 1, fold_bn3_reduce and E > 1
         cb = grp._bwd_cb
         # parameter gradients of the generator's dense layers may still be in flight on the side stream (_FCFn.backward)
         ops.side_stream(dfeat.device).join()
@@ -225,7 +239,7 @@ class _EncoderGroupFn(torch.autograd.Function):
             r = ops.bn_backward_sets(g1, g2_, None if mask_from_z else act, z, st.mean, st.rstd,
                                      [b.weight for b in bns], [b.bias for b in bns] if mask_from_z else None,
                                      dgammas=[tgt(b.weight) for b in bns], dbetas=[tgt(b.bias) for b in bns],
-                                     want_g_out=want_g_out, batch_stats=True, groups=GT, act_bits=act_bits)
+                                     want_g_out=want_g_out, batch_stats=train, groups=GT, act_bits=act_bits)
             return (r[0], r[3]) if want_g_out else r[0]
 
         def dgrad_bn(dy, convs, ksize, bns, st, z):
@@ -233,7 +247,7 @@ class _EncoderGroupFn(torch.autograd.Function):
             and returns the closure that launches the rest (the caller forks the weight gradient in between, so that it
             runs beside the HBM-bound BN pass) and returns dz."""
             wk = _stack_pack(convs, ops.PACK_DGRAD)
-            if not fold_bn_reduce:
+            if not fold:
                 d_a = ops.conv_gemm_grouped(dy, wk, ksize, wgroups=E)
                 return lambda: bn_bwd(bns, st, d_a, None, None, z, mask_from_z=True)
             gm, part = ops.conv_gemm_bnbwd_grouped(dy, wk, ksize, z, st.mean, st.rstd, [b.weight for b in bns],
@@ -287,7 +301,7 @@ class _EncoderGroupFn(torch.autograd.Function):
                 d_a1 = ops.col2im_3x3s2(dcol.view(m2, 9 * planes), nb, hh, ww, planes)
                 dz1 = bn_bwd([b.bn1 for b in blks], st1, d_a1, None, a1, z1, mask_from_z=True)
             wk1 = _stack_pack([b.conv1 for b in blks], ops.PACK_DGRAD)
-            if blks[0].downsample is None and fold_bn3_reduce:
+            if blks[0].downsample is None and fold3:
                 # identity shortcut: this block's input gradient is conv1's data gradient + the masked output gradient,
                 # and the input is the previous block's relu(bn3(z3) + shortcut): that BatchNorm's reduce pass runs here
                 prev = blocks[bidx - 1]
@@ -337,39 +351,44 @@ class EncoderGroup:
         self.grad_targets: Optional[Dict[nn.Parameter, torch.Tensor]] = None
         self._bwd_cb = None  # data-parallel trainer: called with ("pre"|"stage"|"post", stage index) during backward
 
-    def can_run(self, x: torch.Tensor, groups: int) -> bool:
+    def can_run(self, x: torch.Tensor, groups: int, recorded: bool = False) -> bool:
+        """Whether x ([N,3,H,W], `groups` batches stacked along dim 0) runs as one grouped pass.  recorded: autograd
+        records the pass, so an eval-mode pass needs the train-mode kernels' shapes too (the backward runs them)."""
         encs = self.encoders
         if not (x.is_cuda and x.dim() == 4 and x.shape[1] == 3 and x.size(0) % groups == 0):
             return False
         if len({e.training for e in encs}) != 1:
             return False
+        E, n = len(encs), x.size(0)
         h, w = x.shape[2], x.shape[3]
-        if not encs[0].training:
+        if not encs[0].training and not recorded:
             # eval mode: every grouped launch must give each encoder whole tiles of its x.size(0) images (ONE statistic
             # group, the running statistics): the flat GEMMs (stem, 1x1, stride-2 im2col) need a multiple of 128 pixels
             # per encoder, the 3x3 convs a tile geometry with whole images per encoder
             if h < MIN_HW or w < MIN_HW or w > MAX_STEM_W:
                 return False
-            E, n = len(encs), x.size(0)
             for i, (hs, ws) in enumerate(ops.resnet_stage_hw(h, w)):
                 for k in ((1, 3) if i > 0 else (1,)):
                     if ops.conv_geometry(E * n, hs, ws, k, E) is None:
                         return False
             return True
-        if h % 32 or w % 32 or not trainable_shape(x.size(0), h, w):
+        if not trainable_shape(n, h, w):
             return False
-        per_group = x.size(0) // groups
-        return (per_group * (h // 32) * (w // 32)) % 128 == 0
+        # more than one (encoder, statistic group): each needs whole 128-pixel tiles at every stage (layer4 is the
+        # smallest, (H/32) x (W/32) pixels per image)
+        return E * groups == 1 or (n // groups * (h // 32) * (w // 32)) % 128 == 0
 
     def __call__(self, x: torch.Tensor, groups: int = 1, stem_cols=None):
         """Returns features [E, N, 2048, 1, 1]: out[e] == encoders[e].forward_groups(x, groups)."""
-        if not self.can_run(x, groups):
-            raise ops._lib.IrfdError(f"EncoderGroup: shape {tuple(x.shape)} / modes cannot run as one grouped pass")
         encs = self.encoders
-        params = [p for e in encs for p in e._flat_params()]
-        recorded = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
+        recorded = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for e in encs
+                                                                       for p in e.parameters()))
+        if not self.can_run(x, groups, recorded):
+            raise ops._lib.IrfdError(f"EncoderGroup: shape {tuple(x.shape)} / modes cannot run as one grouped pass")
         if not encs[0].training:
-            if recorded:
-                raise ops._lib.IrfdError("EncoderGroup: eval-mode passes with autograd run per encoder")
-            return _group_inference(self, x, stem_cols)
+            if not recorded:
+                return _group_inference(self, x, stem_cols)
+            if len(encs) > 1:
+                raise ops._lib.IrfdError("EncoderGroup: eval-mode passes with autograd run one encoder at a time")
+        params = [p for e in encs for p in e._flat_params()]
         return _EncoderGroupFn.apply(x, self, groups, stem_cols, recorded, *params)

@@ -226,7 +226,8 @@ def conv_gemm_affine(x, wk, ksize, scale, shift, res=None, relu=True, force_bloc
 def conv_gemm_grouped(x, wk, ksize, mode=EPI_PLAIN, wgroups=3, a_shared=False, rows=None, force_block_n=0):
     """One launch for `wgroups` weight sets (the three IRFD encoders).  x [N,H,W,Cin] bf16 stacks the groups' images
     group-major (N = wgroups * images per group); wk [wgroups*Cout, k*k*Cin].  a_shared: x is a 2-D [rows_per_group, K]
-    matrix read by every group (the stem's im2col); the output then has wgroups * rows_per_group rows.
+    matrix read by every group (the stem's im2col); the output then has wgroups * rows_per_group rows (with one group,
+    a plain GEMM over the rows).
     Returns out (mode 0) or (out, stat_sum, stat_sq) (mode 1; partials are [m_tiles, Cout], group-major tiles)."""
     lib = _lib.load()
     _chk(x, BF16, "x")
@@ -252,7 +253,7 @@ def conv_gemm_grouped(x, wk, ksize, mode=EPI_PLAIN, wgroups=3, a_shared=False, r
     nbytes = 2.0 * m * cin / (wgroups if a_shared else 1) + 2.0 * m * cout + 2.0 * wgroups * cin * cout * ksize * ksize
     with _timed("conv_gemm_kernel (tcgen05 fprop/dgrad)", 2.0 * m * cout * cin * ksize * ksize, nbytes):
         _call("irfd_conv_gemm_grouped", x.data_ptr(), n, h, w, cin, wk.data_ptr(), cout, ksize, out.data_ptr(), mode,
-              _ptr(ssum), _ptr(ssq), wgroups, 1 if a_shared else 0, force_block_n, _stream())
+              _ptr(ssum), _ptr(ssq), wgroups, 1 if a_shared and wgroups > 1 else 0, force_block_n, _stream())
     if mode == EPI_STATS:
         return out, ssum, ssq
     return out
@@ -335,8 +336,8 @@ def conv_gemm_affine_grouped(x, wk, ksize, scale, shift, res=None, relu=True, wg
               + 2.0 * wgroups * cin * cout * ksize * ksize)
     with _timed("conv_gemm_kernel (tcgen05 fprop/dgrad)", 2.0 * m * cout * cin * ksize * ksize, nbytes):
         _call("irfd_conv_gemm_affine_grouped", x.data_ptr(), n, h, w, cin, wk.data_ptr(), cout, ksize, out.data_ptr(),
-              scale.data_ptr(), shift.data_ptr(), _ptr(res), int(relu), wgroups, 1 if a_shared else 0, force_block_n,
-              _stream())
+              scale.data_ptr(), shift.data_ptr(), _ptr(res), int(relu), wgroups, 1 if a_shared and wgroups > 1 else 0,
+              force_block_n, _stream())
     return out
 
 
@@ -509,11 +510,6 @@ def bn_finalize(ssum, ssq, count, eps, momentum, running_mean=None, running_var=
     _call("irfd_bn_finalize", ssum.data_ptr(), ssq.data_ptr(), tiles // groups, c, int(count), eps, momentum,
           mean.data_ptr(), rstd.data_ptr(), _ptr(running_mean), _ptr(running_var), running_updates, groups, _stream())
     return mean, rstd
-
-
-def bn_running_update(mean, rstd, eps, count, momentum, running_mean, running_var):
-    _call("irfd_bn_running_update", mean.data_ptr(), rstd.data_ptr(), eps, int(count), momentum,
-          running_mean.data_ptr(), running_var.data_ptr(), mean.numel(), _stream())
 
 
 def bn_eval_rstd(running_var, eps):

@@ -78,8 +78,8 @@ def test_train_step_vs_bf16_faithful_oracle(cuda_device):
 # gradients costs 4e-3), and two implementations that agree to 4e-3 in the forward do not flip the SAME elements.  The
 # encoder bound therefore only catches a gross mis-routing (uncorrelated gradients sit at 1.4); the sharp routing checks
 # of the encoder backward are test_encoder_backward_eval_end_to_end (eval-mode BN, every gradient, median 2.5e-2),
-# test_encoder_backward_train_in_context (every train-mode launch on its own inputs) and
-# test_encoder_group_train_equals_three_passes (lockstep path bit-identical to the per-encoder path).
+# test_gpu_encoder_single.py::test_train_backward_in_context (every train-mode launch on its own inputs) and
+# test_encoder_group_train_equals_three_passes (three-encoder lockstep pass against three one-encoder passes).
 FAITHFUL = {"feat": 8e-3, "img": 1.6e-2, "loss": 3e-3, "running": 5e-3,
             "Gd.synthesis": (1e-2, 8e-2), "Gd.mapping": (8e-2, 0.11), "Gd.noise": (0.1, 0.14), "enc": (0.7, 1.1)}
 
