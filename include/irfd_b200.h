@@ -206,8 +206,14 @@ int irfd_bn_backward_finish_sets(const void* g, const void* z, const float* mean
 /* ------------------------------------------------------------------------------------------------------------------
  * Layout / gather kernels for the strided ResNet convs and pooling (torchvision resnet.py:197-205, 133-137, 241).
  *   irfd_pack_conv_weight: fp32 OIHW -> bf16 GEMM operand. mode 0 fprop [o][tap][i]; 1 dgrad [i][flip(tap)][o];
- *                          2 dcol [(tap,i)][o]; 3 flat [o][kpad] (stem, k = c*49+kh*7+kw, zero padded).
+ *                          2 dcol [(tap,i)][o]; 3 flat [o][kpad] (stem, k = c*49+kh*7+kw, zero padded);
+ *                          4 flat_t [kpad][o], the transpose of 3 (kpad >= i*taps): the stem's dcol = dz @ W operand.
  *   irfd_im2col_stem     : x NCHW fp32 [n,3,h,w] -> col [n*ho*wo][kpad] bf16 (7x7, stride 2, pad 3), w <= 579.
+ *   irfd_col2im_stem     : its adjoint summed over nsets (1..4) column matrices, the image gradient of the encoders
+ *                          that read the same image (replaces autograd's convolution_backward(input) of torchvision
+ *                          resnet.py:197, conv1): dcol [nsets][n*ho*wo][kpad] bf16 (kpad >= 152, 16-byte aligned) ->
+ *                          dx [n,3,h,w] fp32 = sum over e, then kh, then kw of the taps landing on each pixel (a
+ *                          deterministic gather), ho = ceil(h/2), wo = ceil(w/2), any h, w.
  *   irfd_im2col_3x3s2 / irfd_col2im_3x3s2: 3x3 stride-2 pad-1 gather [pix][tap*c + ch] and its adjoint.
  *   The forward gathers (stem, 3x3/2, 1x1/2, max pool) take any h, w and produce ceil(h/2) x ceil(w/2) outputs
  *   (torchvision's sizes); the adjoints (col2im, scatter_add, maxpool_bwd) need even h, w.
@@ -217,6 +223,7 @@ int irfd_bn_backward_finish_sets(const void* g, const void* z, const float* mean
  */
 int irfd_pack_conv_weight(const float* w, void* dst, int o, int i, int taps, int mode, int kpad, irfd_stream_t stream);
 int irfd_im2col_stem(const float* x, void* col, int n, int h, int w, int kpad, irfd_stream_t stream);
+int irfd_col2im_stem(const void* dcol, float* dx, int n, int h, int w, int kpad, int nsets, irfd_stream_t stream);
 int irfd_im2col_3x3s2(const void* a, void* col, int n, int h, int w, int c, irfd_stream_t stream);
 int irfd_col2im_3x3s2(const void* dcol, void* dx, int n, int h, int w, int c, irfd_stream_t stream);
 int irfd_subsample2(const void* a, void* out, int n, int h, int w, int c, irfd_stream_t stream);

@@ -12,6 +12,7 @@ namespace irfd {
 //   mode 1 DGRAD: dst[i][(T-1-tap)*O + o]      = w[o][i][tap]      (spatially flipped, in/out swapped)
 //   mode 2 DCOL : dst[tap*I + i][o]            = w[o][i][tap]      (for dcol = dz @ W)
 //   mode 3 FLAT : dst[o][k], k < kpad          = w[o][k] (k < I*T) else 0   (stem: K = c*49 + kh*7 + kw, padded)
+//   mode 4 FLAT_T: dst[k][o], k < kpad         = w[o][k] (k < I*T) else 0   (stem data gradient: dcol = dz @ W)
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void pack_weight_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ dst, int O, int I, int T,
                                    int mode, int kpad) {
@@ -19,6 +20,12 @@ __global__ void pack_weight_kernel(const float* __restrict__ w, __nv_bfloat16* _
   if (mode == 3) {
     if (idx >= (size_t)O * kpad) return;
     const int o = idx / kpad, k = idx % kpad;
+    dst[idx] = __float2bfloat16(k < I * T ? w[(size_t)o * I * T + k] : 0.f);
+    return;
+  }
+  if (mode == 4) {
+    if (idx >= (size_t)O * kpad) return;
+    const int k = idx / O, o = idx % O;
     dst[idx] = __float2bfloat16(k < I * T ? w[(size_t)o * I * T + k] : 0.f);
     return;
   }
@@ -91,6 +98,109 @@ im2col_stem_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ col,
 #pragma unroll
     for (int t = 0; t < 8; ++t) f[t] = off[t] >= 0 ? srow[off[t] + 2 * ow] : 0.f;
     store8(col + (pix0 + ow) * kpad + v * 8, f);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Stem data gradient, the adjoint of im2col_stem summed over `nsets` column matrices (the encoders that read the same
+// image):  dx[n][c][y][x] = sum_e sum_kh sum_kw dcol[e][(n*Ho + oh)*Wo + ow][(c*7 + kh)*7 + kw]  over the taps with
+// y = 2*oh + kh - 3 and x = 2*ow + kw - 3 inside the stem output (Ho = ceil(H/2)).  A gather in a fixed order (per set
+// the taps in kh, kw order, then the sets in order): no atomics, deterministic.
+// ---------------------------------------------------------------------------------------------------------------
+// A block owns a 32 x 32 tile of output pixels of one image; its taps come from a 19 x 19 window of dcol pixels
+// (oh in [y0/2 - 1, y0/2 + 17]).  Per (set, channel) the window is staged in shared memory: channel c's 49 taps are the
+// seven 16-byte vectors from element 8*floor(49c/8) of the row (column padding from 147 on is never read), and the
+// staged pixel stride is odd in 4-byte words so the 16 distinct pixels a warp reads per tap sit in distinct banks.
+// The next stage's loads are issued before the current stage is summed (ten 16-byte loads in flight per thread).
+// Neighbouring tiles share the 3-pixel halo of their windows; it is read from L2, HBM sees each dcol byte about once.
+constexpr int kC2iTile = 32;                   // output tile edge (even: the window starts at y0/2 - 1)
+constexpr int kC2iWin = kC2iTile / 2 + 3;      // dcol pixels per window edge
+constexpr int kC2iVec = 7;                     // 16-byte vectors per (pixel, channel)
+constexpr int kC2iStride = kC2iVec * 4 + 1;    // staged words per pixel
+constexpr int kC2iThreads = 256;
+constexpr int kC2iPix = kC2iTile * kC2iTile / kC2iThreads;  // output pixels per thread
+constexpr int kC2iStage = kC2iWin * kC2iWin * kC2iVec;      // 16-byte vectors per stage
+constexpr int kC2iLoads = (kC2iStage + kC2iThreads - 1) / kC2iThreads;
+
+__device__ __forceinline__ void c2i_load(uint4 (&q)[kC2iLoads], const __nv_bfloat16* __restrict__ src, int c, int oh0,
+                                         int ow0, int Ho, int Wo, int ld) {
+  const int v0 = c * 49 / 8;
+#pragma unroll
+  for (int j = 0; j < kC2iLoads; ++j) {
+    const int i = threadIdx.x + j * kC2iThreads;
+    const int p = i / kC2iVec, v = i - p * kC2iVec;
+    const int oh = oh0 + p / kC2iWin, ow = ow0 + p % kC2iWin;
+    q[j] = make_uint4(0, 0, 0, 0);  // outside the stem output: the tap falls on padding, contributes 0
+    if (i < kC2iStage && (unsigned)oh < (unsigned)Ho && (unsigned)ow < (unsigned)Wo)
+      q[j] = ldg16(src + ((size_t)oh * Wo + ow) * ld + (v0 + v) * 8);
+  }
+}
+
+__device__ __forceinline__ void c2i_store(const uint4 (&q)[kC2iLoads], uint32_t* stage) {
+#pragma unroll
+  for (int j = 0; j < kC2iLoads; ++j) {
+    const int i = threadIdx.x + j * kC2iThreads;
+    if (i >= kC2iStage) break;
+    const int p = i / kC2iVec, v = i - p * kC2iVec;
+    uint32_t* d = stage + p * kC2iStride + v * 4;
+    d[0] = q[j].x;
+    d[1] = q[j].y;
+    d[2] = q[j].z;
+    d[3] = q[j].w;
+  }
+}
+
+__global__ void __launch_bounds__(kC2iThreads, 2)
+col2im_stem_kernel(const __nv_bfloat16* __restrict__ dcol, float* __restrict__ dx, int N, int H, int W, int ld,
+                   int nsets) {
+  __shared__ uint32_t stage[kC2iWin * kC2iWin * kC2iStride];
+  const __nv_bfloat16* sb = reinterpret_cast<const __nv_bfloat16*>(stage);
+  const int Ho = (H + 1) / 2, Wo = (W + 1) / 2;
+  const int n = blockIdx.z, y0 = blockIdx.y * kC2iTile, x0 = blockIdx.x * kC2iTile;
+  const int oh0 = y0 / 2 - 1, ow0 = x0 / 2 - 1;
+  const size_t set_stride = (size_t)N * Ho * Wo * ld;
+  const __nv_bfloat16* img = dcol + (size_t)n * Ho * Wo * ld;
+  float acc[3][kC2iPix];
+#pragma unroll
+  for (int c = 0; c < 3; ++c)
+#pragma unroll
+    for (int r = 0; r < kC2iPix; ++r) acc[c][r] = 0.f;
+  uint4 q[kC2iLoads];
+  c2i_load(q, img, 0, oh0, ow0, Ho, Wo, ld);
+  for (int e = 0; e < nsets; ++e) {
+#pragma unroll 1
+    for (int c = 0; c < 3; ++c) {
+      __syncthreads();  // the previous stage is consumed
+      c2i_store(q, stage);
+      __syncthreads();
+      const int en = c == 2 ? e + 1 : e;
+      if (en < nsets) c2i_load(q, img + en * set_stride, c == 2 ? 0 : c + 1, oh0, ow0, Ho, Wo, ld);
+      const int off = c * 49 - (c * 49 / 8) * 8;  // tap 0's element in the staged vectors
+#pragma unroll
+      for (int r = 0; r < kC2iPix; ++r) {
+        const int t = threadIdx.x + r * kC2iThreads, ty = t / kC2iTile, tx = t % kC2iTile;
+        // (y + 3 - kh) even; y0 is even, so the first tap has the parity of ty + 1.  Window row of (oh): oh - oh0.
+        float a = 0.f;
+        for (int kh = (ty + 1) & 1; kh < 7; kh += 2) {
+          const int py = (ty + 3 - kh) / 2 + 1;
+          for (int kw = (tx + 1) & 1; kw < 7; kw += 2) {
+            const int px = (tx + 3 - kw) / 2 + 1;
+            a += __bfloat162float(sb[(py * kC2iWin + px) * 2 * kC2iStride + off + kh * 7 + kw]);
+          }
+        }
+        // registers, not a runtime-indexed (local-memory) array
+        acc[0][r] += c == 0 ? a : 0.f;
+        acc[1][r] += c == 1 ? a : 0.f;
+        acc[2][r] += c == 2 ? a : 0.f;
+      }
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < kC2iPix; ++r) {
+    const int t = threadIdx.x + r * kC2iThreads, y = y0 + t / kC2iTile, x = x0 + t % kC2iTile;
+    if (y >= H || x >= W) continue;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) dx[(((size_t)n * 3 + c) * H + y) * W + x] = acc[c][r];
   }
 }
 
@@ -370,8 +480,9 @@ using namespace irfd;
 
 extern "C" int irfd_pack_conv_weight(const float* w, void* dst, int o, int i, int taps, int mode, int kpad,
                                      cudaStream_t stream) {
-  IRFD_CHECK_ARG(w && dst && o > 0 && i > 0 && taps > 0 && mode >= 0 && mode <= 3, "pack_conv_weight: bad argument");
-  const size_t total = mode == 3 ? (size_t)o * kpad : (size_t)o * i * taps;
+  IRFD_CHECK_ARG(w && dst && o > 0 && i > 0 && taps > 0 && mode >= 0 && mode <= 4, "pack_conv_weight: bad argument");
+  IRFD_CHECK_ARG(mode != 4 || kpad >= i * taps, "pack_conv_weight: FLAT_T needs kpad >= %d (got %d)", i * taps, kpad);
+  const size_t total = mode >= 3 ? (size_t)o * kpad : (size_t)o * i * taps;
   pack_weight_kernel<<<GRID1D(total)>>>(w, BF(dst), o, i, taps, mode, kpad);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
@@ -384,6 +495,19 @@ extern "C" int irfd_im2col_stem(const float* x, void* col, int n, int h, int w, 
   IRFD_CHECK_ARG(kStemPixPar * (kpad / 8) <= 256 && (kpad / 8) % 4 == 0, "im2col_stem: kpad a multiple of 32 and <= 256");
   im2col_stem_kernel<<<(unsigned)(n * ((h + 1) / 2)), kStemPixPar * (kpad / 8), smem, stream>>>(x, BF(col), n, h, w,
                                                                                               kpad);
+  IRFD_CHECK_LAUNCH();
+  return IRFD_OK;
+}
+
+extern "C" int irfd_col2im_stem(const void* dcol, float* dx, int n, int h, int w, int kpad, int nsets,
+                                cudaStream_t stream) {
+  IRFD_CHECK_ARG(dcol && dx && ((uintptr_t)dcol & 15) == 0, "col2im_stem: null or unaligned pointer");
+  IRFD_CHECK_ARG(nsets >= 1 && nsets <= 4, "col2im_stem: 1..4 column sets (got %d)", nsets);
+  IRFD_CHECK_ARG(kpad >= 152 && kpad % 8 == 0, "col2im_stem: kpad a multiple of 8 and >= 152 (got %d)", kpad);
+  IRFD_CHECK_ARG(n > 0 && n <= 65535 && h > 0 && w > 0 && h <= 65535 * kC2iTile && w <= 65535 * kC2iTile,
+                 "col2im_stem: bad shape n=%d h=%d w=%d", n, h, w);
+  col2im_stem_kernel<<<dim3((unsigned)((w + kC2iTile - 1) / kC2iTile), (unsigned)((h + kC2iTile - 1) / kC2iTile),
+                            (unsigned)n), kC2iThreads, 0, stream>>>(CBF(dcol), dx, n, h, w, kpad, nsets);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
 }

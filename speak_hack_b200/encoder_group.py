@@ -107,16 +107,18 @@ def _group_inference(grp: "EncoderGroup", x, col0=None):
 
 
 class _EncoderGroupFn(torch.autograd.Function):
-    """forward(x [N,3,H,W] fp32, group, stat_groups, col0, recorded, *params) -> features [E, N, 2048, 1, 1] fp32.
+    """forward(x [N,3,H,W], group, stat_groups, col0, recorded, image_grad, *params) -> features [E, N, 2048, 1, 1] fp32.
 
     Train mode, and eval mode with autograd (E == 1 only); eval-mode forwards without autograd go through
     _group_inference.  params = the encoders' parameters, encoder after encoder, in _flat_params() order.
     In train mode x stacks `stat_groups` independent batches along dim 0 (IRFD: source and target images): BatchNorm
     statistics are per (encoder, group) and each encoder's running buffers are updated group by group, like separate
-    calls.  In eval mode every BatchNorm normalises with its running statistics and no buffer changes."""
+    calls.  In eval mode every BatchNorm normalises with its running statistics and no buffer changes.
+    image_grad: the backward also returns dL/dx, summed over the E encoders (the caller's image came out of a
+    differentiable computation); otherwise x gets no gradient and no launch is spent on it."""
 
     @staticmethod
-    def forward(ctx, x, grp, stat_groups, col0, recorded, *params):
+    def forward(ctx, x, grp, stat_groups, col0, recorded, image_grad, *params):
         encs: List[ResNet50Encoder] = grp.encoders
         E = len(encs)
         train = encs[0].training
@@ -126,8 +128,13 @@ class _EncoderGroupFn(torch.autograd.Function):
         # reentrant-checkpoint semantics of the reference (model.py:84-90, SURVEY Q3): a differentiated pass updates the
         # BN running buffers twice, forward order then reverse order
         U = 2 if (train and recorded and all(getattr(e, "_recompute_bn_update", False) for e in encs)) else 1
+        ctx.image_grad = image_grad and ctx.needs_input_grad[0]
+        ctx.x_dtype = x.dtype
         x = x.contiguous().to(torch.float32)
         n, _, h, w = x.shape
+        # the stem's dcol GEMM gives each encoder whole 128-pixel tiles of the linear geometry (trainable shapes: H and
+        # W are multiples of 32, so n * H/2 * W/2 is a multiple of 256)
+        assert not ctx.image_grad or (n * (h // 2) * (w // 2)) % 128 == 0
 
         def conv(xx, wk, ksize, **kw):
             """Forward conv; in train mode its epilogue also gathers the BatchNorm statistics."""
@@ -203,6 +210,7 @@ class _EncoderGroupFn(torch.autograd.Function):
         if train:  # nn.BatchNorm2d bookkeeping (one fused increment)
             torch._foreach_add_([c for e in encs for c in e._bn_counters()], G * U)
         S["final_hw"] = (cur.shape[1], cur.shape[2])
+        S["x_shape"] = (n, h, w)
         ctx.grp, ctx.S, ctx.G, ctx.train = grp, S, G, train
         return feat.view(E, n, -1, 1, 1)
 
@@ -329,15 +337,23 @@ class _EncoderGroupFn(torch.autograd.Function):
         dz0 = bn_bwd([e[1] for e in encs], st0, d_a0, None, a0, z0, mask_from_z=True)
         # the stem's im2col matrix is shared: every encoder reads the same rows
         wgrad([e[0] for e in encs], col0, dz0.view(-1, 64), 1, x_shared=True, reduce_cin=147, reduce_taps=1)
+        dx = None
+        if ctx.image_grad:
+            # dL/dx of the 7x7/2 stem conv: dcol = dz0 @ W per encoder (one grouped GEMM, [E*P, 192] bf16), then the
+            # col2im gather sums the E encoders' columns onto the image; it runs beside the stem's weight gradient
+            dcol = ops.conv_gemm_grouped(dz0.view(1, 1, -1, 64), _stack_pack([e[0] for e in encs], ops.PACK_FLAT_T, 192),
+                                         1, wgroups=E)
+            dx = ops.col2im_stem(dcol.view(-1, 192), E, *S["x_shape"])
+            if ctx.x_dtype != torch.float32:
+                dx = dx.to(ctx.x_dtype)
         side.join()
         if cb is not None:
             cb("stage", 3)   # the stem (Sequential indices 0, 1)
             cb("post", None)
         ctx.S = None
-        # dL/dx of the stem is not produced (nothing on the IRFD path consumes the image gradient, SURVEY Q2)
         if targets is not None:
-            return (None,) * (5 + sum(len(e._flat_params()) for e in encs))
-        return (None, None, None, None, None) + tuple(grads.get(p) for e in encs for p in e._flat_params())
+            return (dx,) + (None,) * (5 + sum(len(e._flat_params()) for e in encs))
+        return (dx, None, None, None, None, None) + tuple(grads.get(p) for e in encs for p in e._flat_params())
 
 
 class EncoderGroup:
@@ -378,8 +394,11 @@ class EncoderGroup:
         # smallest, (H/32) x (W/32) pixels per image)
         return E * groups == 1 or (n // groups * (h // 32) * (w // 32)) % 128 == 0
 
-    def __call__(self, x: torch.Tensor, groups: int = 1, stem_cols=None):
-        """Returns features [E, N, 2048, 1, 1]: out[e] == encoders[e].forward_groups(x, groups)."""
+    def __call__(self, x: torch.Tensor, groups: int = 1, stem_cols=None, image_grad: Optional[bool] = None):
+        """Returns features [E, N, 2048, 1, 1]: out[e] == encoders[e].forward_groups(x, groups).
+        image_grad: whether the backward returns dL/dx.  Default: when x came out of a differentiable computation
+        (x.grad_fn is set); a leaf image, such as a batch of training data, gets no gradient, as before.  A caller that
+        stacks its images first decides from its own tensors, since the stacking op always has a grad_fn."""
         encs = self.encoders
         recorded = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for e in encs
                                                                        for p in e.parameters()))
@@ -390,5 +409,7 @@ class EncoderGroup:
                 return _group_inference(self, x, stem_cols)
             if len(encs) > 1:
                 raise ops._lib.IrfdError("EncoderGroup: eval-mode passes with autograd run one encoder at a time")
+        if image_grad is None:
+            image_grad = x.grad_fn is not None
         params = [p for e in encs for p in e._flat_params()]
-        return _EncoderGroupFn.apply(x, self, groups, stem_cols, recorded, *params)
+        return _EncoderGroupFn.apply(x, self, groups, stem_cols, recorded, bool(image_grad), *params)

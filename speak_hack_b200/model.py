@@ -52,6 +52,16 @@ def mse_loss(a: torch.Tensor, b: torch.Tensor, scale: float = 1.0) -> torch.Tens
     return _MSEFn.apply(a, b, float(scale))
 
 
+def _stack_images(x_s, x_t):
+    """[x_s; x_t] for the lockstep encoder pass, and whether its backward returns the image gradient: when either image
+    came out of a differentiable computation (the cat itself always has a grad_fn, so the decision is taken here).  A
+    leaf image stacked beside such an image is detached, so that leaf images never receive a gradient."""
+    image_grad = x_s.grad_fn is not None or x_t.grad_fn is not None
+    if image_grad:
+        x_s, x_t = (t if t.grad_fn is not None else t.detach() for t in (x_s, x_t))
+    return torch.cat([x_s, x_t], dim=0), image_grad
+
+
 class IRFD(nn.Module):
     def __init__(self, max_resolution=256):
         super().__init__()
@@ -115,14 +125,14 @@ class IRFD(nn.Module):
         grp = self.encoder_group
         diff = torch.is_grad_enabled() and x_s.requires_grad
         if same and x_s.dim() == 4 and (grp.encoders[0].training or not diff):
-            x = torch.cat([x_s, x_t], dim=0)  # cat keeps requires_grad (SURVEY Q2 semantics)
+            x, image_grad = _stack_images(x_s, x_t)  # cat keeps requires_grad (SURVEY Q2 semantics)
             if grp.can_run(x, 2):
                 B = x_s.size(0)
                 if diff:
                     for enc in grp.encoders:
                         enc._recompute_bn_update = enc.training
                     try:
-                        f = grp(x, 2)
+                        f = grp(x, 2, image_grad=image_grad)
                     finally:
                         for enc in grp.encoders:
                             enc._recompute_bn_update = False
@@ -250,14 +260,19 @@ class _SwapCatStackedFn(torch.autograd.Function):
 def _irfd_forward_static(self: IRFD, x_s, x_t, ctrl):
     """IRFD.forward with the swap / style-mixing decisions taken on the device from `ctrl` (int32 [3]).
     Returns (x_s_recon, x_t_recon, fi_s, fi_t) with fi_* UNswapped (the identity MSE is symmetric in them)."""
-    img, f, b = self.forward_static_stacked(torch.cat([x_s, x_t], dim=0), ctrl)
+    img, f, b = _forward_static_stacked(self, *_stack_images(x_s, x_t), ctrl)
     return img[:b], img[b:], f[0, :b], f[0, b:]
 
 
 def _irfd_forward_static_stacked(self: IRFD, x, ctrl):
     """The whole forward on the stacked batch x = [x_s; x_t] ([2B, 3, H, W]): the three encoders in lockstep (one launch
-    per layer), device-side swap + concat, ONE generator call over the 2B stacked codes.
+    per layer), device-side swap + concat, ONE generator call over the 2B stacked codes.  x receives a gradient when it
+    came out of a differentiable computation (x.grad_fn is set).
     Returns (images [2B, 3, R, R] (source reconstructions first), features [3, 2B, 2048, 1, 1] unswapped, B)."""
+    return _forward_static_stacked(self, x, x.grad_fn is not None, ctrl)
+
+
+def _forward_static_stacked(self: IRFD, x, image_grad, ctrl):
     grp = self.encoder_group
     b = x.size(0) // 2
     diff = torch.is_grad_enabled() and x.requires_grad
@@ -283,7 +298,7 @@ def _irfd_forward_static_stacked(self: IRFD, x, ctrl):
         for enc in grp.encoders:
             enc._recompute_bn_update = enc.training
         try:
-            f = grp(x, 2)
+            f = grp(x, 2, image_grad=image_grad)
         finally:
             for enc in grp.encoders:
                 enc._recompute_bn_update = False

@@ -18,7 +18,7 @@ BF16 = torch.bfloat16
 F32 = torch.float32
 
 EPI_PLAIN, EPI_STATS, EPI_STYLE = 0, 1, 2
-PACK_FPROP, PACK_DGRAD, PACK_DCOL, PACK_FLAT = 0, 1, 2, 3
+PACK_FPROP, PACK_DGRAD, PACK_DCOL, PACK_FLAT, PACK_FLAT_T = 0, 1, 2, 3, 4
 
 # kernels launched through this module since the last reset (bench.py's gpu_launches claim)
 launch_count = 0
@@ -469,7 +469,8 @@ def pack_conv_weights_stacked(ws, mode: int, kpad: int = 0) -> torch.Tensor:
         return hit[1]
     o, i, kh, kw = ws[0].shape
     taps = kh * kw
-    rows, cols = {PACK_FPROP: (o, taps * i), PACK_DGRAD: (i, taps * o), PACK_DCOL: (taps * i, o)}.get(mode, (o, kpad))
+    rows, cols = {PACK_FPROP: (o, taps * i), PACK_DGRAD: (i, taps * o), PACK_DCOL: (taps * i, o),
+                  PACK_FLAT_T: (kpad, o)}.get(mode, (o, kpad))
     dst = torch.empty((len(ws) * rows, cols), dtype=BF16, device=ws[0].device)
     for e, w in enumerate(ws):
         _pack_conv_weight(w, mode, kpad, out=dst[e * rows: (e + 1) * rows])
@@ -487,6 +488,8 @@ def _pack_conv_weight(w: torch.Tensor, mode: int, kpad: int = 0, out: Optional[t
         shape = (i, taps * o)
     elif mode == PACK_DCOL:
         shape = (taps * i, o)
+    elif mode == PACK_FLAT_T:
+        shape = (kpad, o)
     else:
         shape = (o, kpad)
     dst = out if out is not None else torch.empty(shape, dtype=BF16, device=w.device)
@@ -711,6 +714,17 @@ def im2col_stem(x: torch.Tensor, kpad: int = 192) -> torch.Tensor:
     col = torch.empty((n * half_up(h) * half_up(w), kpad), dtype=BF16, device=x.device)
     _call("irfd_im2col_stem", x.data_ptr(), col.data_ptr(), n, h, w, kpad, _stream())
     return col
+
+
+def col2im_stem(dcol: torch.Tensor, nsets: int, n: int, h: int, w: int) -> torch.Tensor:
+    """Adjoint of im2col_stem summed over `nsets` stacked column matrices (the encoders that read the same image):
+    dcol [nsets * n * ceil(h/2) * ceil(w/2), kpad] bf16 -> dx [n, 3, h, w] fp32."""
+    _chk(dcol, BF16, "dcol")
+    if dcol.dim() != 2 or dcol.shape[0] != nsets * n * half_up(h) * half_up(w):
+        raise _lib.IrfdError(f"col2im_stem: dcol {tuple(dcol.shape)} is not {nsets} column matrices of {n}x{h}x{w}")
+    dx = torch.empty((n, 3, h, w), dtype=F32, device=dcol.device)
+    _call("irfd_col2im_stem", dcol.data_ptr(), dx.data_ptr(), n, h, w, dcol.shape[1], nsets, _stream())
+    return dx
 
 
 def im2col_3x3s2(a: torch.Tensor) -> torch.Tensor:
