@@ -66,6 +66,15 @@ int irfd_conv_gemm_m_tiles(int n, int h, int w);
  * Boxed tiles are ordered image-major, then rows, then columns.  Returns IRFD_ERR_INVALID_ARGUMENT for shapes neither
  * geometry serves. */
 int irfd_conv_gemm_geometry(int n, int h, int w, int ksize, int wgroups, int* out_host);
+/* Host-only plan query (no CUDA call beyond the SM count, 148 without a device): which conv_gemm instance the entry
+ * points above launch for these arguments and how its work spreads over the persistent CTAs.  mode 0..5 (4/5: the
+ * BNBWD / BNBWD_RES folds of irfd_conv_gemm_bnbwd[_res]_grouped); a_shared as in irfd_conv_gemm_grouped.  Reads the
+ * IRFD_* environment variables at call time, like the launch.  out_host[9] = {halo (conv_halo_kernel), boxed, BLOCK_N,
+ * cluster (1 single CTA, 2 CTA pair with multicast weights, 3 CTA pair with 2-SM MMAs), per-warp epilogue, m tiles,
+ * n tiles, units, grid}: CTA slot s (s = blockIdx / pair size) serves units s, s + slots, ... with slots = grid / pair
+ * size; a unit is one 256-pixel halo tile x n tile, or (pair size) 128-pixel m tiles x n tile, n tile fastest. */
+int irfd_conv_gemm_plan(int n, int h, int w, int cin, int cout, int ksize, int mode, int wgroups, int a_shared,
+                        int force_block_n, int* out_host);
 int irfd_conv_gemm(const void* x, int n, int h, int w, int cin, const void* wk, int cout, int ksize, void* out,
                    void* out2, int mode, const float* bias, const float* nw, const float* noise, const float* sp1,
                    const float* s1, float* stat_sum, float* stat_sq, int force_block_n, irfd_stream_t stream);
@@ -121,6 +130,12 @@ long long irfd_wgrad_workspace_bytes_grouped(int n, int h, int w, int cin, int c
 int irfd_conv_wgrad_grouped(const void* x, const void* dy, int n, int h, int w, int cin, int cout, int ksize,
                             float* const* dw, float beta, int reduce_cin, int reduce_taps, int groups, int x_shared,
                             void* workspace, long long workspace_bytes, irfd_stream_t stream);
+/* Host-only plan query of irfd_conv_wgrad_grouped with the same shape arguments (groups = 1: irfd_conv_wgrad); reads
+ * IRFD_WGRAD_HALO at call time.  out_host[7] = {halo (wgrad_halo_kernel), BLOCK_N, splits, k blocks per split, k blocks
+ * per group (64 pixels per-tap, 128 halo), GEMM grid, reduce kernel (0 transpose<9>, 1 transpose<1>, 2 reduce<1>,
+ * 3 reduce<4>, 4 reduce<8>)}.  Split s covers k blocks [s * per split, min((s + 1) * per split, k blocks)). */
+int irfd_conv_wgrad_plan(int n, int h, int w, int cin, int cout, int ksize, int groups, int x_shared, int reduce_cin,
+                         int reduce_taps, int* out_host);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * BatchNorm2d around the encoder convs (torch.nn.BatchNorm2d in torchvision Bottleneck, resnet.py:143-164).

@@ -1030,7 +1030,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 // ------------------------------------------------------------------------------------------------
 template <int BLOCK_N, int MODE, int CL = 1, bool MMA2 = false, bool BOX = false>
 static int launch_conv_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo, const CUtensorMap& mo2,
-                            const ConvGemmArgs& a, cudaStream_t stream) {
+                            const ConvGemmArgs& a, int grid, cudaStream_t stream) {
   using Cfg = GemmCfg<BLOCK_N, MODE>;
   static bool configured = false;
   auto kern = conv_gemm_kernel<BLOCK_N, MODE, CL, MMA2, BOX>;
@@ -1042,9 +1042,6 @@ static int launch_conv_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const 
     }
     configured = true;
   }
-  const int units = (a.num_m_tiles / CL) * a.num_n_tiles;
-  const int slots = num_sms() / CL;
-  const int grid = (units < slots ? units : slots) * CL;
   if (CL == 1) {
     kern<<<grid, kNumThreads, Cfg::SMEM_BYTES, stream>>>(ma, mb, mo, mo2, a);
   } else {
@@ -1068,21 +1065,21 @@ static int launch_conv_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const 
 
 template <int MODE>
 static int dispatch_block_n(int block_n, const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo,
-                            const CUtensorMap& mo2, const ConvGemmArgs& a, cudaStream_t stream, int cluster = 1) {
+                            const CUtensorMap& mo2, const ConvGemmArgs& a, int grid, int cluster, cudaStream_t stream) {
   if constexpr (MODE == EPI_PLAIN || MODE == EPI_STATS || MODE == EPI_BNBWD) {
     if (cluster == 3) {  // CTA pairs with 2-SM MMAs
-      if (block_n == 128) return launch_conv_gemm<128, MODE, 2, true>(ma, mb, mo, mo2, a, stream);
-      if (block_n == 256) return launch_conv_gemm<256, MODE, 2, true>(ma, mb, mo, mo2, a, stream);
+      if (block_n == 128) return launch_conv_gemm<128, MODE, 2, true>(ma, mb, mo, mo2, a, grid, stream);
+      if (block_n == 256) return launch_conv_gemm<256, MODE, 2, true>(ma, mb, mo, mo2, a, grid, stream);
     }
   }
   if (cluster >= 2) {
-    if (block_n == 128) return launch_conv_gemm<128, MODE, 2>(ma, mb, mo, mo2, a, stream);
-    if (block_n == 256) return launch_conv_gemm<256, MODE, 2>(ma, mb, mo, mo2, a, stream);
+    if (block_n == 128) return launch_conv_gemm<128, MODE, 2>(ma, mb, mo, mo2, a, grid, stream);
+    if (block_n == 256) return launch_conv_gemm<256, MODE, 2>(ma, mb, mo, mo2, a, grid, stream);
   }
   switch (block_n) {
-    case 64: return launch_conv_gemm<64, MODE>(ma, mb, mo, mo2, a, stream);
-    case 128: return launch_conv_gemm<128, MODE>(ma, mb, mo, mo2, a, stream);
-    case 256: return launch_conv_gemm<256, MODE>(ma, mb, mo, mo2, a, stream);
+    case 64: return launch_conv_gemm<64, MODE>(ma, mb, mo, mo2, a, grid, stream);
+    case 128: return launch_conv_gemm<128, MODE>(ma, mb, mo, mo2, a, grid, stream);
+    case 256: return launch_conv_gemm<256, MODE>(ma, mb, mo, mo2, a, grid, stream);
   }
   set_last_error("bad BLOCK_N %d", block_n);
   return IRFD_ERR_INVALID_ARGUMENT;
@@ -1090,11 +1087,11 @@ static int dispatch_block_n(int block_n, const CUtensorMap& ma, const CUtensorMa
 
 template <int MODE>
 static int dispatch_box(int block_n, const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo,
-                        const ConvGemmArgs& a, cudaStream_t stream) {
+                        const ConvGemmArgs& a, int grid, cudaStream_t stream) {
   switch (block_n) {
-    case 64: return launch_conv_gemm<64, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
-    case 128: return launch_conv_gemm<128, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
-    case 256: return launch_conv_gemm<256, MODE, 1, false, true>(ma, mb, mo, mo, a, stream);
+    case 64: return launch_conv_gemm<64, MODE, 1, false, true>(ma, mb, mo, mo, a, grid, stream);
+    case 128: return launch_conv_gemm<128, MODE, 1, false, true>(ma, mb, mo, mo, a, grid, stream);
+    case 256: return launch_conv_gemm<256, MODE, 1, false, true>(ma, mb, mo, mo, a, grid, stream);
   }
   set_last_error("bad BLOCK_N %d", block_n);
   return IRFD_ERR_INVALID_ARGUMENT;
@@ -1103,7 +1100,7 @@ static int dispatch_box(int block_n, const CUtensorMap& ma, const CUtensorMap& m
 
 template <int BLOCK_N, int MODE>
 static int launch_conv_halo(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo, const CUtensorMap& mo2,
-                            const ConvGemmArgs& a, const HaloArgs& h, cudaStream_t stream) {
+                            const ConvGemmArgs& a, const HaloArgs& h, int grid, cudaStream_t stream) {
   using Cfg = HaloCfg<BLOCK_N, MODE>;
   static bool configured = false;
   auto kern = conv_halo_kernel<BLOCK_N, MODE>;
@@ -1115,7 +1112,6 @@ static int launch_conv_halo(const CUtensorMap& ma, const CUtensorMap& mb, const 
     }
     configured = true;
   }
-  const int grid = h.total_tiles < num_sms() ? h.total_tiles : num_sms();
   kern<<<grid, kHaloThreads, Cfg::SMEM_BYTES, stream>>>(ma, mb, mo, mo2, a, h);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
@@ -1123,9 +1119,10 @@ static int launch_conv_halo(const CUtensorMap& ma, const CUtensorMap& mb, const 
 
 template <int MODE>
 static int dispatch_halo(int block_n, const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mo,
-                         const CUtensorMap& mo2, const ConvGemmArgs& a, const HaloArgs& h, cudaStream_t stream) {
-  if (block_n == 64) return launch_conv_halo<64, MODE>(ma, mb, mo, mo2, a, h, stream);
-  return launch_conv_halo<128, MODE>(ma, mb, mo, mo2, a, h, stream);
+                         const CUtensorMap& mo2, const ConvGemmArgs& a, const HaloArgs& h, int grid,
+                         cudaStream_t stream) {
+  if (block_n == 64) return launch_conv_halo<64, MODE>(ma, mb, mo, mo2, a, h, grid, stream);
+  return launch_conv_halo<128, MODE>(ma, mb, mo, mo2, a, h, grid, stream);
 }
 
 // IRFD_GEMM_CLUSTER: 1 = CTA pairs with multicast weight tiles where the layer allows it, 0 (default) = never.
@@ -1264,12 +1261,20 @@ struct BnBwdFold {  // EPI_BNBWD / EPI_BNBWD_RES operands (see ConvGemmArgs)
   int stat_groups;
 };
 
-static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const void* wk, int cout, int ksize, void* out,
-                          void* out2, void* out_lo, int mode, const float* bias, const float* nw, const float* noise,
-                          const float* sp1, const float* s1, float* stat_sum, float* stat_sq, const void* res, int relu,
-                          int force_block_n, cudaStream_t stream, int wgroups = 1, int a_shared = 0,
-                          const BnBwdFold* fold = nullptr) {
-  IRFD_CHECK_ARG(x && wk && out, "conv_gemm: null pointer");
+// Which kernel instance a conv_gemm call launches and how its work spreads over the persistent CTAs: the one place the
+// selection lives (conv_gemm_impl launches what it says; irfd_conv_gemm_plan exports it).  Reads the IRFD_* variables
+// at call time and makes no CUDA call beyond num_sms().
+struct ConvPlan {
+  TileGeom geo;
+  int use_halo, block_n, cluster, warp_epi;
+  int num_m_tiles, num_n_tiles;
+  int units;  // work units the CTAs walk (unit u: CTA slot u % slots, slots = grid / pair size, pair size 2 when
+              // cluster > 1): halo tiles of 256 pixels x n tiles, or pair-size groups of 128-pixel m tiles x n tiles
+  int grid;   // CTAs launched
+};
+
+static int conv_gemm_plan(int n, int h, int w, int cin, int cout, int ksize, int mode, int wgroups, int a_shared,
+                          int force_block_n, ConvPlan* pl) {
   IRFD_CHECK_ARG(ksize == 1 || ksize == 3, "conv_gemm: ksize must be 1 or 3 (got %d)", ksize);
   IRFD_CHECK_ARG(cin % 64 == 0 && cin > 0, "conv_gemm: Cin must be a multiple of 64 (got %d)", cin);
   IRFD_CHECK_ARG(cout % 64 == 0 && cout > 0, "conv_gemm: Cout must be a multiple of 64 (got %d)", cout);
@@ -1281,7 +1286,7 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
   IRFD_CHECK_ARG(wgroups == 1 || (mode != EPI_STYLE), "conv_gemm: weight groups are not available in STYLE mode");
   IRFD_CHECK_ARG(!a_shared || (ksize == 1 && wgroups > 1), "conv_gemm: a shared A operand needs ksize 1 and groups > 1");
 
-  TileGeom geo;
+  TileGeom& geo = pl->geo;
   {
     const int rc = tile_geometry(n, h, w, ksize, wgroups, a_shared, &geo);
     if (rc != IRFD_OK) return rc;
@@ -1290,13 +1295,92 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
   IRFD_CHECK_ARG(!boxed || mode == EPI_PLAIN || mode == EPI_AFFINE,
                  "conv_gemm: n=%d h=%d w=%d (ksize %d) needs box tiles, which serve the plain and affine epilogues only "
                  "(mode %d)", n, h, w, ksize, mode);
+  const int H = geo.H, W = geo.W;
+  const int num_m_tiles = boxed ? geo.tiles_w * geo.tiles_h * geo.tiles_n : (m_total + 127) / 128;
+  const int wg_tiles = wgroups > 1 ? num_m_tiles / wgroups : 0x7fffffff;
+  const int a_mod_tiles = a_shared ? num_m_tiles / wgroups : 0;
+  pl->num_m_tiles = num_m_tiles;
+  pl->warp_epi = (mode != EPI_STYLE && !boxed && m_total % 128 == 0 && warp_epi_mode() != 0) ? 1 : 0;
+
+  int block_n = force_block_n;
+  if (block_n == 0) {
+    block_n = 64;
+    const int cands[3] = {256, 128, 64};
+    for (int i = 0; i < 3; ++i) {
+      if (cout % cands[i] == 0 && (long long)num_m_tiles * (cout / cands[i]) >= num_sms()) {
+        block_n = cands[i];
+        break;
+      }
+    }
+    // small-M layers: 128-wide tiles on >= 2/3 of the SMs beat 64-wide tiles on all of them (measured,
+    // scripts/exp_blockn.py: 512->512 3x3 @8^2 x64 images 41 -> 29 us, 2048->512 1x1 23.5 -> 18.4 us)
+    if (block_n == 64 && cout % 128 == 0 && (long long)num_m_tiles * (cout / 128) * 3 >= 2ll * num_sms()) block_n = 128;
+  }
+  IRFD_CHECK_ARG((block_n == 64 || block_n == 128 || block_n == 256) && cout % block_n == 0,
+                 "conv_gemm: BLOCK_N %d incompatible with Cout %d", block_n, cout);
+  // halo-reuse kernel: 3x3, rows of >= 128 pixels, Cout of one 64/128-wide tile (the fabric-bound generator layers)
+  const int hmode = halo_mode();
+  const bool use_halo = hmode != 0 && !boxed && mode != EPI_BNBWD && mode != EPI_BNBWD_RES && wgroups == 1 && ksize == 3 && W % 128 == 0 && H % 2 == 0 &&
+                        (cout == 64 || cout == 128) &&
+                        (force_block_n == 0 || force_block_n == cout);
+  if (use_halo) block_n = cout;
+  pl->use_halo = use_halo ? 1 : 0;
+  pl->block_n = block_n;
+  pl->num_n_tiles = cout / block_n;
+  // CTA pairs (multicast weight tiles): two consecutive m tiles must belong to the same weight group / A matrix
+  int cluster = 1;
+  if (!use_halo && !boxed && (cluster_mode() != 0 || mma2_mode() != 0) && block_n >= 128 && num_m_tiles % 2 == 0 &&
+      (wgroups == 1 || wg_tiles % 2 == 0) && (a_mod_tiles == 0 || a_mod_tiles % 2 == 0))
+    cluster = (mma2_mode() != 0 && pl->warp_epi && (mode == EPI_PLAIN || mode == EPI_STATS || mode == EPI_BNBWD)) ? 3 : 2;
+  pl->cluster = cluster;
+  if (use_halo) {  // one CTA per SM, each walking 256-pixel tiles (two image rows x 128 columns)
+    pl->units = geo.NB * (H / 2) * (W / 128) * pl->num_n_tiles;
+    pl->grid = pl->units < num_sms() ? pl->units : num_sms();
+  } else {
+    const int cl = cluster > 1 ? 2 : 1;
+    pl->units = (num_m_tiles / cl) * pl->num_n_tiles;
+    const int slots = num_sms() / cl;
+    pl->grid = (pl->units < slots ? pl->units : slots) * cl;
+  }
+  return IRFD_OK;
+}
+
+extern "C" int irfd_conv_gemm_plan(int n, int h, int w, int cin, int cout, int ksize, int mode, int wgroups,
+                                   int a_shared, int force_block_n, int* out_host) {
+  IRFD_CHECK_ARG(out_host != nullptr, "conv_gemm_plan: null output");
+  ConvPlan pl;
+  const int rc = conv_gemm_plan(n, h, w, cin, cout, ksize, mode, wgroups, a_shared, force_block_n, &pl);
+  if (rc != IRFD_OK) return rc;
+  const int v[9] = {pl.use_halo, pl.geo.boxed, pl.block_n, pl.cluster, pl.warp_epi,
+                    pl.num_m_tiles, pl.num_n_tiles, pl.units, pl.grid};
+  for (int i = 0; i < 9; ++i) out_host[i] = v[i];
+  return IRFD_OK;
+}
+
+static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const void* wk, int cout, int ksize, void* out,
+                          void* out2, void* out_lo, int mode, const float* bias, const float* nw, const float* noise,
+                          const float* sp1, const float* s1, float* stat_sum, float* stat_sq, const void* res, int relu,
+                          int force_block_n, cudaStream_t stream, int wgroups = 1, int a_shared = 0,
+                          const BnBwdFold* fold = nullptr) {
+  IRFD_CHECK_ARG(x && wk && out, "conv_gemm: null pointer");
+  ConvPlan pl;
+  {
+    const int rc = conv_gemm_plan(n, h, w, cin, cout, ksize, mode, wgroups, a_shared, force_block_n, &pl);
+    if (rc != IRFD_OK) return rc;
+  }
+  const TileGeom& geo = pl.geo;
+  const bool boxed = geo.boxed != 0;
+  const int m_total = n * h * w;
   const int H = geo.H, W = geo.W, NB = geo.NB;
   const int tw = geo.tw, th = geo.th, tn = geo.tn;
+  const bool use_halo = pl.use_halo != 0;
+  const int block_n = pl.block_n, cluster = pl.cluster;
 
   ConvGemmArgs a;
   a.M_total = m_total;
   a.N_total = cout;
-  a.num_m_tiles = boxed ? geo.tiles_w * geo.tiles_h * geo.tiles_n : (m_total + 127) / 128;
+  a.num_m_tiles = pl.num_m_tiles;
+  a.num_n_tiles = pl.num_n_tiles;
   a.box_tw = tw;
   a.box_th = th;
   a.box_tn = tn;
@@ -1320,7 +1404,7 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     IRFD_CHECK_ARG(h * w >= 64, "conv_gemm: STYLE mode needs >= 64 pixels per image");
   }
   if (mode == EPI_STATS) IRFD_CHECK_ARG(stat_sum && stat_sq, "conv_gemm: STATS mode needs stat buffers");
-  a.warp_epi = (mode != EPI_STYLE && !boxed && m_total % 128 == 0 && warp_epi_mode() != 0) ? 1 : 0;
+  a.warp_epi = pl.warp_epi;
   a.bn_z = nullptr;
   a.bn_mean = a.bn_rstd = nullptr;
   for (int i = 0; i < 4; ++i) a.bn_gamma[i] = a.bn_beta[i] = nullptr;
@@ -1350,35 +1434,6 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     a.sg_tiles = a.num_m_tiles / fold->stat_groups;
   }
 
-  int block_n = force_block_n;
-  if (block_n == 0) {
-    block_n = 64;
-    const int cands[3] = {256, 128, 64};
-    for (int i = 0; i < 3; ++i) {
-      if (cout % cands[i] == 0 && (long long)a.num_m_tiles * (cout / cands[i]) >= num_sms()) {
-        block_n = cands[i];
-        break;
-      }
-    }
-    // small-M layers: 128-wide tiles on >= 2/3 of the SMs beat 64-wide tiles on all of them (measured,
-    // scripts/exp_blockn.py: 512->512 3x3 @8^2 x64 images 41 -> 29 us, 2048->512 1x1 23.5 -> 18.4 us)
-    if (block_n == 64 && cout % 128 == 0 && (long long)a.num_m_tiles * (cout / 128) * 3 >= 2ll * num_sms()) block_n = 128;
-  }
-  IRFD_CHECK_ARG((block_n == 64 || block_n == 128 || block_n == 256) && cout % block_n == 0,
-                 "conv_gemm: BLOCK_N %d incompatible with Cout %d", block_n, cout);
-  // halo-reuse kernel: 3x3, rows of >= 128 pixels, Cout of one 64/128-wide tile (the fabric-bound generator layers)
-  const int hmode = halo_mode();
-  const bool use_halo = hmode != 0 && !boxed && mode != EPI_BNBWD && mode != EPI_BNBWD_RES && wgroups == 1 && ksize == 3 && W % 128 == 0 && H % 2 == 0 &&
-                        (cout == 64 || cout == 128) &&
-                        (force_block_n == 0 || force_block_n == cout);
-  if (use_halo) block_n = cout;
-  a.num_n_tiles = cout / block_n;
-  // CTA pairs (multicast weight tiles): two consecutive m tiles must belong to the same weight group / A matrix
-  int cluster = 1;
-  if (!use_halo && !boxed && (cluster_mode() != 0 || mma2_mode() != 0) && block_n >= 128 && a.num_m_tiles % 2 == 0 &&
-      (wgroups == 1 || a.wg_tiles % 2 == 0) && (a.a_mod_tiles == 0 || a.a_mod_tiles % 2 == 0))
-    cluster = (mma2_mode() != 0 && a.warp_epi && (mode == EPI_PLAIN || mode == EPI_STATS || mode == EPI_BNBWD)) ? 3 : 2;
-
   CUtensorMap ma, mb, mo, mo2;
   {
     const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)H, (uint64_t)NB};
@@ -1406,8 +1461,8 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     const uint32_t box[4] = {64, (uint32_t)tw, (uint32_t)th, (uint32_t)tn};
     const int rc = make_tmap_bf16(&mo, out, 4, dims, str, box, true);
     if (rc) return rc;
-    if (mode == EPI_PLAIN) return dispatch_box<EPI_PLAIN>(block_n, ma, mb, mo, a, stream);
-    return dispatch_box<EPI_AFFINE>(block_n, ma, mb, mo, a, stream);
+    if (mode == EPI_PLAIN) return dispatch_box<EPI_PLAIN>(block_n, ma, mb, mo, a, pl.grid, stream);
+    return dispatch_box<EPI_AFFINE>(block_n, ma, mb, mo, a, pl.grid, stream);
   }
   {
     const uint64_t dims[2] = {(uint64_t)cout, (uint64_t)m_total};
@@ -1427,22 +1482,22 @@ static int conv_gemm_impl(const void* x, int n, int h, int w, int cin, const voi
     HaloArgs hargs;
     hargs.wsegs = W / 128;
     hargs.hpairs = H / 2;
-    hargs.total_tiles = NB * hargs.hpairs * hargs.wsegs * a.num_n_tiles;
+    hargs.total_tiles = pl.units;
     switch (mode) {
-      case EPI_PLAIN: return dispatch_halo<EPI_PLAIN>(block_n, ma, mb, mo, mo2, a, hargs, stream);
-      case EPI_STATS: return dispatch_halo<EPI_STATS>(block_n, ma, mb, mo, mo2, a, hargs, stream);
-      case EPI_STYLE: return dispatch_halo<EPI_STYLE>(block_n, ma, mb, mo, mo2, a, hargs, stream);
-      case EPI_AFFINE: return dispatch_halo<EPI_AFFINE>(block_n, ma, mb, mo, mo2, a, hargs, stream);
+      case EPI_PLAIN: return dispatch_halo<EPI_PLAIN>(block_n, ma, mb, mo, mo2, a, hargs, pl.grid, stream);
+      case EPI_STATS: return dispatch_halo<EPI_STATS>(block_n, ma, mb, mo, mo2, a, hargs, pl.grid, stream);
+      case EPI_STYLE: return dispatch_halo<EPI_STYLE>(block_n, ma, mb, mo, mo2, a, hargs, pl.grid, stream);
+      case EPI_AFFINE: return dispatch_halo<EPI_AFFINE>(block_n, ma, mb, mo, mo2, a, hargs, pl.grid, stream);
     }
     return IRFD_ERR_INVALID_ARGUMENT;
   }
   switch (mode) {
-    case EPI_PLAIN: return dispatch_block_n<EPI_PLAIN>(block_n, ma, mb, mo, mo2, a, stream, cluster);
-    case EPI_STATS: return dispatch_block_n<EPI_STATS>(block_n, ma, mb, mo, mo2, a, stream, cluster);
-    case EPI_STYLE: return dispatch_block_n<EPI_STYLE>(block_n, ma, mb, mo, mo2, a, stream, cluster);
-    case EPI_AFFINE: return dispatch_block_n<EPI_AFFINE>(block_n, ma, mb, mo, mo2, a, stream, cluster);
-    case EPI_BNBWD: return dispatch_block_n<EPI_BNBWD>(block_n, ma, mb, mo, mo2, a, stream, cluster);
-    case EPI_BNBWD_RES: return dispatch_block_n<EPI_BNBWD_RES>(block_n, ma, mb, mo, mo2, a, stream, cluster);
+    case EPI_PLAIN: return dispatch_block_n<EPI_PLAIN>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
+    case EPI_STATS: return dispatch_block_n<EPI_STATS>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
+    case EPI_STYLE: return dispatch_block_n<EPI_STYLE>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
+    case EPI_AFFINE: return dispatch_block_n<EPI_AFFINE>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
+    case EPI_BNBWD: return dispatch_block_n<EPI_BNBWD>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
+    case EPI_BNBWD_RES: return dispatch_block_n<EPI_BNBWD_RES>(block_n, ma, mb, mo, mo2, a, pl.grid, cluster, stream);
   }
   return IRFD_ERR_INVALID_ARGUMENT;
 }

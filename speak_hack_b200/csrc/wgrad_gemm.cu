@@ -290,29 +290,43 @@ wgrad_reduce_transpose_kernel(const float* __restrict__ partial, WgDst dws, int 
   }
 }
 
-// few splits: one thread per output; many splits (1x1 layers, halo kernel: up to 148): 8 lanes share the walk
-static void launch_wgrad_reduce(const float* partial, const WgDst& dws, int groups, int splits, int K_total, int N_total,
-                                int cin, int taps, float beta, cudaStream_t stream) {
+// The split-K reduce kernel launch_wgrad_reduce runs (irfd_conv_wgrad_plan reports it): few splits, one thread per
+// output; many splits (1x1 layers, halo kernel: up to 148), 8 lanes share the walk.
+enum { kWgRedTranspose9 = 0, kWgRedTranspose1 = 1, kWgRed1 = 2, kWgRed4 = 3, kWgRed8 = 4 };
+
+static int wgrad_reduce_kind(int splits, int K_total, int N_total, int cin, int taps) {
   const size_t total = (size_t)K_total * N_total;
   // the transposing kernel needs whole 32 x 32 tiles and the plain k = tap*cin + c layout (no padded K tail)
   const bool tileable = cin % 32 == 0 && N_total % 32 == 0 && K_total == cin * taps && (taps == 9 || taps == 1);
-  if (splits <= 6 && tileable && total >= (size_t)1 << 18) {
-    const dim3 grid(N_total / 32, cin / 32, groups);
-    if (taps == 9)
-      wgrad_reduce_transpose_kernel<9><<<grid, 256, 0, stream>>>(partial, dws, splits, K_total, N_total, cin, beta);
-    else
-      wgrad_reduce_transpose_kernel<1><<<grid, 256, 0, stream>>>(partial, dws, splits, K_total, N_total, cin, beta);
-    return;
+  if (splits <= 6 && tileable && total >= (size_t)1 << 18) return taps == 9 ? kWgRedTranspose9 : kWgRedTranspose1;
+  if (splits <= 6) return kWgRed1;
+  return splits <= 24 ? kWgRed4 : kWgRed8;
+}
+
+static void launch_wgrad_reduce(const float* partial, const WgDst& dws, int groups, int splits, int K_total, int N_total,
+                                int cin, int taps, float beta, cudaStream_t stream) {
+  const size_t total = (size_t)K_total * N_total;
+  switch (wgrad_reduce_kind(splits, K_total, N_total, cin, taps)) {
+    case kWgRedTranspose9:
+      wgrad_reduce_transpose_kernel<9><<<dim3(N_total / 32, cin / 32, groups), 256, 0, stream>>>(
+          partial, dws, splits, K_total, N_total, cin, beta);
+      break;
+    case kWgRedTranspose1:
+      wgrad_reduce_transpose_kernel<1><<<dim3(N_total / 32, cin / 32, groups), 256, 0, stream>>>(
+          partial, dws, splits, K_total, N_total, cin, beta);
+      break;
+    case kWgRed1:
+      wgrad_reduce_kernel<1><<<dim3((unsigned)((total + 255) / 256), groups), 256, 0, stream>>>(
+          partial, dws, splits, K_total, N_total, cin, taps, beta);
+      break;
+    case kWgRed4:
+      wgrad_reduce_kernel<4><<<dim3((unsigned)((total + 63) / 64), groups), 256, 0, stream>>>(
+          partial, dws, splits, K_total, N_total, cin, taps, beta);
+      break;
+    default:
+      wgrad_reduce_kernel<8><<<dim3((unsigned)((total + 31) / 32), groups), 256, 0, stream>>>(
+          partial, dws, splits, K_total, N_total, cin, taps, beta);
   }
-  if (splits <= 6)
-    wgrad_reduce_kernel<1><<<dim3((unsigned)((total + 255) / 256), groups), 256, 0, stream>>>(
-        partial, dws, splits, K_total, N_total, cin, taps, beta);
-  else if (splits <= 24)
-    wgrad_reduce_kernel<4><<<dim3((unsigned)((total + 63) / 64), groups), 256, 0, stream>>>(
-        partial, dws, splits, K_total, N_total, cin, taps, beta);
-  else
-    wgrad_reduce_kernel<8><<<dim3((unsigned)((total + 31) / 32), groups), 256, 0, stream>>>(
-        partial, dws, splits, K_total, N_total, cin, taps, beta);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -561,7 +575,7 @@ static bool wgrad_halo_plan(int n, int h, int w, int cin, int cout, int ksize, W
 }
 
 template <int BLOCK_N>
-static int launch_wgrad(const CUtensorMap& mx, const CUtensorMap& mdy, const WgradArgs& a, cudaStream_t stream) {
+static int launch_wgrad(const CUtensorMap& mx, const CUtensorMap& mdy, const WgradArgs& a, int grid, cudaStream_t stream) {
   using Cfg = WgCfg<BLOCK_N>;
   static bool configured = false;
   auto kern = wgrad_gemm_kernel<BLOCK_N>;
@@ -573,7 +587,6 @@ static int launch_wgrad(const CUtensorMap& mx, const CUtensorMap& mdy, const Wgr
     }
     configured = true;
   }
-  const int grid = a.groups * a.num_pairs * a.num_n_tiles * a.splits;
   kern<<<grid, kWgThreads, Cfg::SMEM_BYTES, stream>>>(mx, mdy, a);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
@@ -637,18 +650,64 @@ extern "C" long long irfd_wgrad_workspace_bytes_grouped(int n, int h, int w, int
   return wgrad_ws_bytes(1, 1, (int)(((long long)n * h * w) / groups), cin, cout, ksize, groups);  // 2-D row matrices
 }
 
-static int conv_wgrad_impl(const void* x, const void* dy, int n, int h, int w, int cin, int cout, int ksize,
-                           const WgDst& dws, int groups, int x_shared, float beta, int reduce_cin, int reduce_taps,
-                           void* workspace, long long workspace_bytes, cudaStream_t stream) {
-  // n, h, w: geometry of ONE group
-  IRFD_CHECK_ARG(x && dy && workspace, "conv_wgrad: null pointer");
+// Which kernels a weight-gradient call launches (halo or per-tap GEMM, then one split-K reduce): the one place the
+// selection lives (conv_wgrad_impl launches what it says; irfd_conv_wgrad_plan exports it).  n, h, w: ONE group.
+struct WgradSel {
+  bool halo;
+  WgHaloArgs ha;  // halo
+  WgradArgs a;    // per-tap
+  int block_n, splits, kb_per_split, num_kb, grid;
+  int red_cin, red_taps, reduce_kind;
+};
+
+static int wgrad_select(int n, int h, int w, int cin, int cout, int ksize, int groups, int x_shared, int reduce_cin,
+                        int reduce_taps, WgradSel* s) {
   IRFD_CHECK_ARG(ksize == 1 || ksize == 3, "conv_wgrad: ksize must be 1 or 3");
   IRFD_CHECK_ARG(cin % 64 == 0 && cout % 64 == 0, "conv_wgrad: channels must be multiples of 64");
   IRFD_CHECK_ARG(!x_shared || ksize == 1, "conv_wgrad: a shared x operand needs ksize 1");
   const long long m_group = (long long)n * h * w;
   IRFD_CHECK_ARG(groups == 1 || m_group % 128 == 0, "conv_wgrad: grouped launches need 128-pixel multiples per group");
-  WgHaloArgs ha;
-  if (!x_shared && wgrad_halo_plan(n, h, w, cin, cout, ksize, &ha, groups)) {
+  s->halo = !x_shared && wgrad_halo_plan(n, h, w, cin, cout, ksize, &s->ha, groups);
+  int K_total, N_total, taps;
+  if (s->halo) {
+    s->block_n = 64;
+    s->splits = s->ha.splits;
+    s->kb_per_split = s->ha.kb_per_split;
+    s->num_kb = s->ha.num_kb;
+    s->grid = groups * s->ha.chunks * s->ha.num_n_tiles * s->ha.splits;
+    K_total = s->ha.K_total;
+    N_total = s->ha.N_total;
+    taps = 9;
+  } else {
+    wgrad_plan(n, h, w, cin, cout, ksize, &s->a, &s->block_n, groups);
+    s->a.x_shared = x_shared;
+    s->splits = s->a.splits;
+    s->kb_per_split = s->a.kb_per_split;
+    s->num_kb = s->a.num_kb;
+    s->grid = groups * s->a.num_pairs * s->a.num_n_tiles * s->a.splits;
+    K_total = s->a.K_total;
+    N_total = s->a.N_total;
+    taps = s->a.taps;
+  }
+  s->red_cin = reduce_cin > 0 ? reduce_cin : cin;
+  s->red_taps = reduce_cin > 0 ? reduce_taps : taps;
+  s->reduce_kind = wgrad_reduce_kind(s->splits, K_total, N_total, s->red_cin, s->red_taps);
+  return IRFD_OK;
+}
+
+static int conv_wgrad_impl(const void* x, const void* dy, int n, int h, int w, int cin, int cout, int ksize,
+                           const WgDst& dws, int groups, int x_shared, float beta, int reduce_cin, int reduce_taps,
+                           void* workspace, long long workspace_bytes, cudaStream_t stream) {
+  // n, h, w: geometry of ONE group
+  IRFD_CHECK_ARG(x && dy && workspace, "conv_wgrad: null pointer");
+  WgradSel sel;
+  {
+    const int rc = wgrad_select(n, h, w, cin, cout, ksize, groups, x_shared, reduce_cin, reduce_taps, &sel);
+    if (rc != IRFD_OK) return rc;
+  }
+  const long long m_group = (long long)n * h * w;
+  if (sel.halo) {
+    WgHaloArgs& ha = sel.ha;
     IRFD_CHECK_ARG(workspace_bytes >= (long long)groups * ha.splits * ha.K_total * ha.N_total * 4,
                    "conv_wgrad: workspace too small");
     ha.partial = reinterpret_cast<float*>(workspace);
@@ -676,17 +735,15 @@ static int conv_wgrad_impl(const void* x, const void* dy, int n, int h, int w, i
       }
       configured = true;
     }
-    wgrad_halo_kernel<<<groups * ha.chunks * ha.num_n_tiles * ha.splits, kWgThreads, kWhSmem, stream>>>(mx, mdy, ha);
+    wgrad_halo_kernel<<<sel.grid, kWgThreads, kWhSmem, stream>>>(mx, mdy, ha);
     IRFD_CHECK_LAUNCH();
-    launch_wgrad_reduce(ha.partial, dws, groups, ha.splits, ha.K_total, ha.N_total, reduce_cin > 0 ? reduce_cin : cin,
-                        reduce_cin > 0 ? reduce_taps : 9, beta, stream);
+    launch_wgrad_reduce(ha.partial, dws, groups, ha.splits, ha.K_total, ha.N_total, sel.red_cin, sel.red_taps, beta,
+                        stream);
     IRFD_CHECK_LAUNCH();
     return IRFD_OK;
   }
-  WgradArgs a;
-  int block_n;
-  wgrad_plan(n, h, w, cin, cout, ksize, &a, &block_n, groups);
-  a.x_shared = x_shared;
+  WgradArgs& a = sel.a;
+  const int block_n = sel.block_n;
   IRFD_CHECK_ARG(workspace_bytes >= (long long)groups * a.splits * a.K_total * a.N_total * 4,
                  "conv_wgrad: workspace too small");
   a.partial = reinterpret_cast<float*>(workspace);
@@ -731,13 +788,12 @@ static int conv_wgrad_impl(const void* x, const void* dy, int n, int h, int w, i
   }
   int rc;
   switch (block_n) {
-    case 64: rc = launch_wgrad<64>(mx, mdy, a, stream); break;
-    case 128: rc = launch_wgrad<128>(mx, mdy, a, stream); break;
-    default: rc = launch_wgrad<256>(mx, mdy, a, stream); break;
+    case 64: rc = launch_wgrad<64>(mx, mdy, a, sel.grid, stream); break;
+    case 128: rc = launch_wgrad<128>(mx, mdy, a, sel.grid, stream); break;
+    default: rc = launch_wgrad<256>(mx, mdy, a, sel.grid, stream); break;
   }
   if (rc) return rc;
-  launch_wgrad_reduce(a.partial, dws, groups, a.splits, a.K_total, a.N_total, reduce_cin > 0 ? reduce_cin : cin,
-                      reduce_cin > 0 ? reduce_taps : a.taps, beta, stream);
+  launch_wgrad_reduce(a.partial, dws, groups, a.splits, a.K_total, a.N_total, sel.red_cin, sel.red_taps, beta, stream);
   IRFD_CHECK_LAUNCH();
   return IRFD_OK;
 }
@@ -756,6 +812,18 @@ extern "C" int irfd_conv_wgrad(const void* x, const void* dy, int n, int h, int 
 // group-major (n = TOTAL images, n % groups == 0; 2-D row matrices pass n = 1, h = 1, w = total rows); dw is a HOST
 // array of `groups` device pointers (one OIHW fp32 gradient each).  x_shared != 0 (ksize 1): x holds ONE group's rows,
 // read by every group (the stem's im2col matrix); n/h/w then describe dy.
+// n, h, w of a grouped call (TOTAL images, or a 2-D row matrix [1, 1, rows]) -> the geometry of one group
+static int wgrad_group_shape(int n, int h, int w, int groups, int* ng, int* hg, int* wg) {
+  *ng = n; *hg = h; *wg = w;
+  if (n % groups == 0) {
+    *ng = n / groups;
+  } else {  // 2-D row matrix [1, 1, rows, K]
+    IRFD_CHECK_ARG(n == 1 && h == 1 && w % groups == 0, "conv_wgrad_grouped: rows do not split into groups");
+    *wg = w / groups;
+  }
+  return IRFD_OK;
+}
+
 extern "C" int irfd_conv_wgrad_grouped(const void* x, const void* dy, int n, int h, int w, int cin, int cout, int ksize,
                                        float* const* dw, float beta, int reduce_cin, int reduce_taps, int groups,
                                        int x_shared, void* workspace, long long workspace_bytes, cudaStream_t stream) {
@@ -763,13 +831,25 @@ extern "C" int irfd_conv_wgrad_grouped(const void* x, const void* dy, int n, int
   WgDst dws;
   for (int i = 0; i < kMaxWgGroups; ++i) dws.p[i] = i < groups ? dw[i] : nullptr;
   for (int i = 0; i < groups; ++i) IRFD_CHECK_ARG(dws.p[i] != nullptr, "conv_wgrad_grouped: null gradient pointer");
-  int ng = n, hg = h, wg = w;
-  if (n % groups == 0) {
-    ng = n / groups;
-  } else {  // 2-D row matrix [1, 1, rows, K]
-    IRFD_CHECK_ARG(n == 1 && h == 1 && w % groups == 0, "conv_wgrad_grouped: rows do not split into groups");
-    wg = w / groups;
-  }
+  int ng, hg, wg;
+  const int rc = wgrad_group_shape(n, h, w, groups, &ng, &hg, &wg);
+  if (rc != IRFD_OK) return rc;
   return conv_wgrad_impl(x, dy, ng, hg, wg, cin, cout, ksize, dws, groups, x_shared, beta, reduce_cin, reduce_taps,
                          workspace, workspace_bytes, stream);
+}
+
+// Host-only query of the kernels irfd_conv_wgrad_grouped launches for these arguments (groups = 1: irfd_conv_wgrad).
+extern "C" int irfd_conv_wgrad_plan(int n, int h, int w, int cin, int cout, int ksize, int groups, int x_shared,
+                                    int reduce_cin, int reduce_taps, int* out_host) {
+  IRFD_CHECK_ARG(out_host != nullptr, "conv_wgrad_plan: null output");
+  IRFD_CHECK_ARG(groups >= 1 && groups <= kMaxWgGroups, "conv_wgrad_plan: 1..4 groups");
+  int ng, hg, wg;
+  int rc = wgrad_group_shape(n, h, w, groups, &ng, &hg, &wg);
+  if (rc != IRFD_OK) return rc;
+  WgradSel sel;
+  rc = wgrad_select(ng, hg, wg, cin, cout, ksize, groups, x_shared, reduce_cin, reduce_taps, &sel);
+  if (rc != IRFD_OK) return rc;
+  const int v[7] = {sel.halo ? 1 : 0, sel.block_n, sel.splits, sel.kb_per_split, sel.num_kb, sel.grid, sel.reduce_kind};
+  for (int i = 0; i < 7; ++i) out_host[i] = v[i];
+  return IRFD_OK;
 }

@@ -689,6 +689,31 @@ def conv_geometry(n: int, h: int, w: int, ksize: int, wgroups: int = 1):
     return tuple(out)
 
 
+CONV_PLAN_FIELDS = ("halo", "boxed", "block_n", "cluster", "warp_epi", "m_tiles", "n_tiles", "units", "grid")
+WGRAD_PLAN_FIELDS = ("halo", "block_n", "splits", "kb_per_split", "num_kb", "grid", "reduce")
+WGRAD_REDUCE_KERNELS = ("transpose<9>", "transpose<1>", "reduce<1>", "reduce<4>", "reduce<8>")
+
+
+def conv_plan(n: int, h: int, w: int, cin: int, cout: int, ksize: int, mode: int, wgroups: int = 1,
+              a_shared: bool = False, force_block_n: int = 0):
+    """Kernel instance and CTA work split a conv_gemm call with these arguments launches (irfd_conv_gemm_plan,
+    host-only, reads the IRFD_* variables now): dict over CONV_PLAN_FIELDS, or None when the call would be refused."""
+    out = (ctypes.c_int * len(CONV_PLAN_FIELDS))()
+    rc = _lib.load().irfd_conv_gemm_plan(n, h, w, cin, cout, ksize, mode, wgroups, 1 if a_shared else 0,
+                                         force_block_n, out)
+    return dict(zip(CONV_PLAN_FIELDS, out)) if rc == _lib.IRFD_OK else None
+
+
+def wgrad_plan(n: int, h: int, w: int, cin: int, cout: int, ksize: int, groups: int = 1, x_shared: bool = False,
+               reduce_cin: int = 0, reduce_taps: int = 0):
+    """Kernels a conv_wgrad(_grouped) call launches (irfd_conv_wgrad_plan, host-only): dict over WGRAD_PLAN_FIELDS
+    with n = TOTAL images, or None when the call would be refused."""
+    out = (ctypes.c_int * len(WGRAD_PLAN_FIELDS))()
+    rc = _lib.load().irfd_conv_wgrad_plan(n, h, w, cin, cout, ksize, groups, 1 if x_shared else 0, reduce_cin,
+                                          reduce_taps, out)
+    return dict(zip(WGRAD_PLAN_FIELDS, out)) if rc == _lib.IRFD_OK else None
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 # layout / pooling
 # ----------------------------------------------------------------------------------------------------------------------
