@@ -360,6 +360,30 @@ long long irfd_bias_lrelu_bwd_workspace_bytes(long long rows, int c);
 int irfd_bias_lrelu_bwd(const void* g, const void* y, void* dz, float* dbias, long long rows, int c, void* workspace,
                         long long workspace_bytes, irfd_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * Spectral normalisation of every layer of one discriminator call (torch.nn.utils.spectral_norm, one power iteration,
+ * styleganv1.py:643-654).  Layer i: W = weight_orig [rows_host[i], cols_host[i]] fp32 (conv: [Cout, Cin*k*k]),
+ * u [rows] and v [cols] its weight_u / weight_v buffers.  w, u, v, w_sn, g, dw are HOST arrays of `nlayers` (1..32)
+ * device pointers, read at call time.  Every reduction has a fixed order (no atomics): results are bit-reproducible.
+ *   irfd_spectral_norm_fwd: power_iteration != 0 (train mode), in torch's order and in place on u and v:
+ *                             v = W^T u / max(|W^T u|, eps);  u = W v / max(|W v|, eps);  sigma = u . (W v)
+ *                           power_iteration == 0 (eval mode): sigma = u . (W v) with the stored u, v.
+ *                           w_sn[i] = W / sigma (fp32, W's layout); sigma [nlayers] fp32.  u_save [sum rows] /
+ *                           v_save [sum cols] (optional) receive the u and v this call used, layer after layer.
+ *                           3 launches (train) or 2 (eval).
+ *   irfd_spectral_norm_bwd: u, v, sigma as saved by the forward; g[i] = dL/dW_sn:
+ *                           dw[i] = (g - <g, W_sn> u v^T) / sigma  (u, v are constants, as in torch).  2 launches.
+ *   workspace >= irfd_spectral_norm_workspace_bytes(rows_host, cols_host, nlayers) bytes (either direction).
+ */
+long long irfd_spectral_norm_workspace_bytes(const int* rows_host, const int* cols_host, int nlayers);
+int irfd_spectral_norm_fwd(const float* const* w, float* const* u, float* const* v, float* const* w_sn, float* u_save,
+                           float* v_save, float* sigma, const int* rows_host, const int* cols_host, int nlayers,
+                           int power_iteration, float eps, void* workspace, long long workspace_bytes,
+                           irfd_stream_t stream);
+int irfd_spectral_norm_bwd(const float* const* g, const float* const* w_sn, const float* u, const float* v,
+                           const float* sigma, float* const* dw, const int* rows_host, const int* cols_host,
+                           int nlayers, void* workspace, long long workspace_bytes, irfd_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -24,12 +24,16 @@ image's.  `D.r1_penalty(x)` is the same computation fused into one node (it skip
 generic double backward cannot know it does not need).
 
 Spectral normalisation itself (one power iteration on each [Cout, Cin*k*k] matrix, styleganv1.py:643-654 via
-torch.nn.utils.spectral_norm) stays in its torch hook: it is parameter preparation — a few mat-vecs per layer, like the
-fp32 -> bf16 weight repack — and keeping the hook keeps `weight_u / weight_v` updates and the backward through sigma
-exactly the reference's.  There is no PyTorch composition of the network in this module: inputs the kernels cannot
-take (CPU tensors, other resolutions, channel counts that are not multiples of 64) raise.
+torch.nn.utils.spectral_norm) runs in its torch hook by default, which keeps `weight_u / weight_v` updates and the
+backward through sigma exactly the reference's.  Inside `D.native_spectral_norm()` (the graphed discriminator step,
+trainer.IRFDDiscriminatorStep(use_cuda_graph=True)) the same computation runs on the sm_100a kernels instead, all
+layers of a call in 3 launches forward and 2 backward (_SpectralNormFn).  There is no PyTorch composition of the
+network in this module: inputs the kernels cannot take (CPU tensors, other resolutions, channel counts that are not
+multiples of 64) raise.
 """
 from __future__ import annotations
+
+import contextlib
 
 import numpy as np
 import torch
@@ -57,6 +61,29 @@ def _normalized_weight(m: nn.Module) -> torch.Tensor:
     for hook in m._forward_pre_hooks.values():
         hook(m, None)
     return m.weight
+
+
+class _SpectralNormFn(torch.autograd.Function):
+    """forward(power_iteration, n, weight_orig x n, weight_u x n, weight_v x n) -> n spectrally normalised weights
+    W_sn = weight_orig / sigma, on the sm_100a kernels (ops.spectral_norm_fwd): in train mode one power iteration per
+    layer updates weight_u / weight_v in place, as torch.nn.utils.spectral_norm's hook does.  Backward treats u and v as
+    constants, like the hook (it differentiates weight_orig / sigma with u, v cloned):
+    dL/dweight_orig = (G - <G, W_sn> u v^T) / sigma."""
+
+    @staticmethod
+    def forward(ctx, power_iteration, n, *tensors):
+        ws, us, vs = tensors[:n], tensors[n: 2 * n], tensors[2 * n:]
+        outs, u_save, v_save, sigma = ops.spectral_norm_fwd(ws, us, vs, power_iteration)
+        ctx.n = n
+        ctx.save_for_backward(u_save, v_save, sigma, *outs)
+        return tuple(outs)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, *grads):
+        u_save, v_save, sigma, *outs = ctx.saved_tensors
+        dws = ops.spectral_norm_bwd(grads, outs, u_save, v_save, sigma)
+        return (None, None) + tuple(dws) + (None,) * (2 * ctx.n)
 
 
 _ones_cache = {}
@@ -297,14 +324,33 @@ class StyleDiscriminator(nn.Module):
             return False
         return all(b.conv1.weight_orig.shape[0] % 64 == 0 and b.conv2.weight_orig.shape[0] % 64 == 0 for b in self.blocks)
 
-    def _weights_and_biases(self):
+    def _sn_modules(self):
         mods = [self.fromrgb]
         for blk in self.blocks:
             mods += [blk.conv1, blk.conv2]
-        mods += [self.final_conv, self.dense0, self.dense1]
+        return mods + [self.final_conv, self.dense0, self.dense1]
+
+    @contextlib.contextmanager
+    def native_spectral_norm(self):
+        """Within this context every call normalises its weights with the sm_100a spectral-norm kernels (one
+        _SpectralNormFn node per call) instead of the torch hooks: same u / v updates and gradients, a fixed number of
+        launches, capturable in a CUDA graph.  Outside it the hooks run, exactly as in the reference."""
+        prev, self._native_sn = self.__dict__.get("_native_sn", False), True
+        try:
+            yield self
+        finally:
+            self._native_sn = prev
+
+    def _weights_and_biases(self):
+        mods = self._sn_modules()
+        if self.__dict__.get("_native_sn", False):
+            ws = _SpectralNormFn.apply(self.training, len(mods), *[m.weight_orig for m in mods],
+                                       *[m.weight_u for m in mods], *[m.weight_v for m in mods])
+        else:
+            ws = [_normalized_weight(m) for m in mods]
         wb = []
-        for m in mods:
-            wb += [_normalized_weight(m), m.bias]
+        for m, w in zip(mods, ws):
+            wb += [w, m.bias]
         return wb
 
     def r1_penalty(self, real_img):

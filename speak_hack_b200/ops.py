@@ -977,6 +977,60 @@ def bias_lrelu_bwd(g, y):
     return dz, dbias
 
 
+def _sn_shapes(ws):
+    """(rows, cols) host int arrays of the [rows, cols] matrix views of spectrally normalised weights."""
+    n = len(ws)
+    rows = (ctypes.c_int * n)(*[w.shape[0] for w in ws])
+    cols = (ctypes.c_int * n)(*[w.numel() // w.shape[0] for w in ws])
+    return rows, cols
+
+
+def spectral_norm_fwd(ws, us, vs, power_iteration: bool, eps: float = 1e-12):
+    """One spectral-norm pass over the layers of a discriminator call.  ws: weight_orig tensors (fp32, any rank, matrix
+    view [shape[0], rest]); us / vs: their weight_u / weight_v buffers, updated in place when power_iteration.
+    Returns ([W_sn per layer, shaped like ws], u_save [sum rows], v_save [sum cols], sigma [layers]): the u and v the
+    normalisation used, for spectral_norm_bwd."""
+    lib = _lib.load()
+    for w, u, v in zip(ws, us, vs):
+        for t, name in ((w, "weight_orig"), (u, "weight_u"), (v, "weight_v")):
+            _chk(t, F32, name)
+        if u.numel() != w.shape[0] or v.numel() != w.numel() // w.shape[0]:
+            raise _lib.IrfdError(f"spectral_norm_fwd: u {tuple(u.shape)} / v {tuple(v.shape)} do not match the "
+                                 f"[{w.shape[0]}, {w.numel() // w.shape[0]}] matrix of weight {tuple(w.shape)}")
+    dev = ws[0].device
+    rows, cols = _sn_shapes(ws)
+    flat = torch.empty(sum(w.numel() for w in ws), dtype=F32, device=dev)
+    outs, off = [], 0
+    for w in ws:
+        outs.append(flat[off: off + w.numel()].view(w.shape))
+        off += w.numel()
+    u_save = torch.empty(sum(rows), dtype=F32, device=dev)
+    v_save = torch.empty(sum(cols), dtype=F32, device=dev)
+    sigma = torch.empty(len(ws), dtype=F32, device=dev)
+    wsp = workspace(lib.irfd_spectral_norm_workspace_bytes(rows, cols, len(ws)), dev)
+    _call("irfd_spectral_norm_fwd", _ptr_array(ws), _ptr_array(us), _ptr_array(vs), _ptr_array(outs),
+          u_save.data_ptr(), v_save.data_ptr(), sigma.data_ptr(), rows, cols, len(ws), 1 if power_iteration else 0,
+          float(eps), wsp.data_ptr(), wsp.numel(), _stream(), launches=3 if power_iteration else 2)
+    return outs, u_save, v_save, sigma
+
+
+def spectral_norm_bwd(gs, w_sns, u_save, v_save, sigma):
+    """dL/dweight_orig per layer from dL/dW_sn (gs), the forward's outputs and the u / v / sigma it saved."""
+    lib = _lib.load()
+    gs = [g.contiguous() for g in gs]
+    for g, w in zip(gs, w_sns):
+        _chk(g, F32, "grad")
+        if g.shape != w.shape:
+            raise _lib.IrfdError(f"spectral_norm_bwd: gradient {tuple(g.shape)} != weight {tuple(w.shape)}")
+    dev = gs[0].device
+    rows, cols = _sn_shapes(w_sns)
+    dws = [torch.empty_like(w) for w in w_sns]
+    wsp = workspace(lib.irfd_spectral_norm_workspace_bytes(rows, cols, len(gs)), dev)
+    _call("irfd_spectral_norm_bwd", _ptr_array(gs), _ptr_array(w_sns), u_save.data_ptr(), v_save.data_ptr(),
+          sigma.data_ptr(), _ptr_array(dws), rows, cols, len(gs), wsp.data_ptr(), wsp.numel(), _stream(), launches=2)
+    return dws
+
+
 # ----------------------------------------------------------------------------------------------------------------------
 # fp32 dense layers
 # ----------------------------------------------------------------------------------------------------------------------

@@ -98,6 +98,78 @@ class _BCELogitsFn(torch.autograd.Function):
         return g * (torch.sigmoid(x) - ctx.target) / x.numel(), None
 
 
+class StepGraph:
+    """The graph-mode plumbing the generator step (IRFDTrainer) and the discriminator step (IRFDDiscriminatorStep)
+    share: the reference's CPU-generator draws uploaded as a device control tensor, the device step counter of the
+    captured Adam, and capture with rollback of the warm-up passes."""
+
+    def __init__(self, model: IRFD, device: torch.device):
+        self.model = model
+        self.device = device
+        self.ctrl = torch.zeros(3, dtype=torch.int32, device=device)
+        # ring of pinned control buffers: an async H2D copy reads its pinned source when the STREAM reaches it, and the
+        # CPU runs several graph replays ahead, so a slot is rewritten only after the copy that read it has completed
+        self._ring = ([(torch.zeros(3, dtype=torch.int32).pin_memory(), torch.cuda.Event()) for _ in range(8)]
+                      if device.type == "cuda" else [])
+        self._slot = 0
+        self.last_ctrl = None
+        self.step_dev = torch.zeros(1, dtype=torch.int32, device=device)
+
+    def draw_ctrl(self):
+        """The reference's CPU-generator draws of one IRFD.forward, in its order: swap (model.py:98), then per Gd call
+        rand(1) and, when mixing, randint(1, L) (styleganv1.py:548, 552)."""
+        gd = self.model.Gd
+        L = gd.synthesis.num_layers
+        vals = [int(torch.randint(0, 3, (1,)).item())]
+        for g in range(2):
+            cut = L
+            if gd.training and gd.style_mixing_prob > 0:
+                if torch.rand(1) < gd.style_mixing_prob:
+                    cut = int(torch.randint(1, L, (1,)).item())
+            vals.append(cut)
+        self.upload_ctrl(vals)
+
+    def upload_ctrl(self, vals):
+        host, ev = self._ring[self._slot]
+        self._slot = (self._slot + 1) % len(self._ring)
+        ev.synchronize()  # no-op unless the CPU is a whole ring ahead of the device
+        host[0], host[1], host[2] = vals
+        self.ctrl.copy_(host, non_blocking=True)
+        ev.record()
+        self.last_ctrl = tuple(vals)
+
+    def capture(self, owner, body, state):
+        """Capture body() (one step of `owner`) into a CUDA graph.  Two warm-up passes run first (allocator, lazy
+        function attributes, pack caches); they are real steps, so everything they mutate is put back: the tensors in
+        `state`, owner.step_count, the device step counter and both RNG streams.  Returns (graph, launches)."""
+        dev = self.device
+        self.step_dev.fill_(owner.step_count)
+        snap = [t.clone() for t in state]
+        snap_step = owner.step_count
+        cpu_rng, cuda_rng = torch.get_rng_state(), torch.cuda.get_rng_state(dev)
+        side = torch.cuda.Stream(dev)
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            for _ in range(2):
+                self.draw_ctrl()
+                body()
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        before = ops.launch_count
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            body()
+        launches = ops.launch_count - before
+        # the captured pass was only recorded, not executed; the warm-up passes are rolled back
+        for t, c in zip(state, snap):
+            t.copy_(c)
+        owner.step_count = snap_step
+        self.step_dev.fill_(snap_step)
+        torch.set_rng_state(cpu_rng)
+        torch.cuda.set_rng_state(cuda_rng, dev)
+        return graph, launches
+
+
 class IRFDTrainer:
     def __init__(self, model: IRFD, lr: float = 2e-4, betas=(0.9, 0.999), eps: float = 1e-8,
                  grad_clip: Optional[float] = None, encoder_grads: bool = True, use_cuda_graph: bool = False,
@@ -132,15 +204,9 @@ class IRFDTrainer:
         self.use_cuda_graph = use_cuda_graph
         self.graph: Optional[torch.cuda.CUDAGraph] = None
         self.graph_launches = 0
-        self.ctrl = torch.zeros(3, dtype=torch.int32, device=self.device)
-        # ring of pinned control buffers: an async H2D copy reads its pinned source when the STREAM reaches it, and the
-        # CPU runs several graph replays ahead, so a slot is rewritten only after the copy that read it has completed
-        self._ctrl_ring = ([(torch.zeros(3, dtype=torch.int32).pin_memory(), torch.cuda.Event()) for _ in range(8)]
-                           if self.device.type == "cuda" else [])
-        self._ctrl_slot = 0
+        self._graphed = StepGraph(model, self.device)
+        self.ctrl, self.step_dev = self._graphed.ctrl, self._graphed.step_dev
         self._graph_key = None
-        self.last_ctrl = None
-        self.step_dev = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._static = None
 
     # ---------------------------------------------------------------------------------------------- shared pieces
@@ -231,29 +297,6 @@ class IRFDTrainer:
         return loss.detach()
 
     # ---------------------------------------------------------------------------------------------- static-graph step
-    def _draw_ctrl(self):
-        """The reference's CPU-generator draws, in its order: swap (model.py:98), then per Gd call rand(1) and, when
-        mixing, randint(1, L) (styleganv1.py:548, 552)."""
-        gd = self.model.Gd
-        L = gd.synthesis.num_layers
-        vals = [int(torch.randint(0, 3, (1,)).item())]
-        for g in range(2):
-            cut = L
-            if gd.training and gd.style_mixing_prob > 0:
-                if torch.rand(1) < gd.style_mixing_prob:
-                    cut = int(torch.randint(1, L, (1,)).item())
-            vals.append(cut)
-        self._upload_ctrl(vals)
-
-    def _upload_ctrl(self, vals):
-        host, ev = self._ctrl_ring[self._ctrl_slot]
-        self._ctrl_slot = (self._ctrl_slot + 1) % len(self._ctrl_ring)
-        ev.synchronize()  # no-op unless the CPU is a whole ring ahead of the device
-        host[0], host[1], host[2] = vals
-        self.ctrl.copy_(host, non_blocking=True)
-        ev.record()
-        self.last_ctrl = tuple(vals)
-
     def _static_body(self):
         x_all, loss_out, lid_out, lrec_out = self._static
         b = x_all.size(0) // 2
@@ -298,43 +341,13 @@ class IRFDTrainer:
                             torch.zeros((), device=dev), torch.zeros((), device=dev))
 
     def _capture(self, x_s, x_t):
-        dev = self.device
         self._ensure_static(x_s)
         b = x_s.size(0)
         self._static[0][:b].copy_(x_s)
         self._static[0][b:].copy_(x_t)
-        self.step_dev.fill_(self.step_count)
-        # The warm-up passes below are real steps; snapshot everything they mutate (Gd parameters, Adam moments, BN
-        # running buffers, step counters, both RNG streams) and put it back, so capturing is invisible to training.
-        snap = [t.clone() for t in (self.flat, self.m, self.v)]
         bufs = [bf for e in self.encoders for bf in e.buffers()]
         bufs += [bf for bf in self.model.D.buffers()] if self.adv_weight is not None else []
-        snap_bufs = [bf.clone() for bf in bufs]
-        snap_step = self.step_count
-        cpu_rng, cuda_rng = torch.get_rng_state(), torch.cuda.get_rng_state(dev)
-        side = torch.cuda.Stream(dev)
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):  # warm-up on a side stream (allocator, lazy function attributes, pack cache)
-            for _ in range(2):
-                self._draw_ctrl()
-                self._static_body()
-        torch.cuda.current_stream().wait_stream(side)
-        torch.cuda.synchronize()
-        before = ops.launch_count
-        graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph):
-            self._static_body()
-        launches = ops.launch_count - before
-        # the captured pass was only recorded, not executed; the warm-up passes are rolled back
-        for t, c in zip((self.flat, self.m, self.v), snap):
-            t.copy_(c)
-        for bf, c in zip(bufs, snap_bufs):
-            bf.copy_(c)
-        self.step_count = snap_step
-        self.step_dev.fill_(snap_step)
-        torch.set_rng_state(cpu_rng)
-        torch.cuda.set_rng_state(cuda_rng, dev)
-        return graph, launches
+        return self._graphed.capture(self, self._static_body, [self.flat, self.m, self.v] + bufs)
 
     def _graph_state(self, x_s):
         """What a captured graph bakes in besides the buffers it owns: the train/eval mode of every sub-network, the
@@ -355,7 +368,7 @@ class IRFDTrainer:
         b = x_s.size(0)
         self._static[0][:b].copy_(x_s, non_blocking=True)   # straight into the stacked static batch: no torch.cat
         self._static[0][b:].copy_(x_t, non_blocking=True)
-        self._draw_ctrl()
+        self._graphed.draw_ctrl()
         self.graph.replay()
         self.step_count += 1
         ops.launch_count += self.graph_launches
@@ -369,7 +382,7 @@ class IRFDTrainer:
         b = x_s.size(0)
         self._static[0][:b].copy_(x_s, non_blocking=True)
         self._static[0][b:].copy_(x_t, non_blocking=True)
-        self._draw_ctrl()
+        self._graphed.draw_ctrl()
         self.step_dev.fill_(self.step_count)
         self._static_body()
         return self._static[1]
@@ -481,11 +494,22 @@ class IRFDDiscriminatorStep:
         loss_D = real + fake + r1_weight * R1 -> backward -> Adam(lr 5e-5) on D.parameters()   (train.py:347)
 
     Every D call is its own forward (one spectral-norm power iteration each, like the reference's six calls).  D's
-    parameters and gradients are views of flat fp32 buffers, so zero_grad and Adam are one launch each.  Eager launches
-    (no CUDA graph: the spectral-norm hooks are torch code); the G step is the graphed path."""
+    parameters and gradients are views of flat fp32 buffers, so zero_grad and Adam are one launch each.  By default the
+    step launches eagerly and D normalises its weights in the torch spectral-norm hooks.
+
+    `use_cuda_graph=True` captures the whole step into one CUDA graph: the six D calls, each with its own power
+    iteration on the native spectral-norm kernels (D.native_spectral_norm()), the instance noise (drawn in the graph
+    from the CUDA generator), the no-grad IRFD forward as IRFD.forward_static_stacked (source and target stacked, ONE
+    generator call over both, so the generator's noise planes are drawn over the stacked batch), BCE, the fused R1
+    node, backward, the data-parallel gradient average and Adam.  The swap and style-mixing draws are taken from the
+    CPU generator every step in the order IRFD.forward takes them (StepGraph.draw_ctrl), so a loop that alternates G
+    and D steps sees the same CPU RNG stream in either mode.  The generator's bf16 weight repacks run inside the graph
+    (the G step's Adam rewrites its weights between D steps); the encoders' are graph constants, so a change of their
+    weights (load_state_dict), of any module's mode, of the batch shape, style_mixing_prob, lr, betas, eps, r1_weight
+    or noise_std recaptures."""
 
     def __init__(self, model: IRFD, lr: float = 5e-5, betas=(0.9, 0.999), eps: float = 1e-8, r1_weight: float = 1.0,
-                 noise_std: float = 0.1):
+                 noise_std: float = 0.1, use_cuda_graph: bool = False):
         self.model = model
         self.lr, self.betas, self.eps = lr, betas, eps
         self.r1_weight, self.noise_std = r1_weight, noise_std
@@ -496,11 +520,31 @@ class IRFDDiscriminatorStep:
         self.v = torch.zeros_like(self.flat)
         self.step_count = 0
         self.last = None
+        # static-graph state
+        self.use_cuda_graph = use_cuda_graph
+        self.device = self.flat.device
+        self.encoders = [model.Ei, model.Ee, model.Ep]
+        self._gd_conv_weights = [p for p in model.Gd.parameters() if p.dim() == 4 and p.shape[-1] == 3]
+        self._graphed = StepGraph(model, self.device)
+        self.ctrl, self.step_dev = self._graphed.ctrl, self._graphed.step_dev
+        self.buckets = GradBuckets(self.device)
+        self.world = self.buckets.world
+        self.graph: Optional[torch.cuda.CUDAGraph] = None
+        self.graph_launches = 0
+        self.captures = 0
+        self._graph_key = None
+        self._static = None
 
     def _noisy(self, x):
         return torch.add(x.detach(), torch.randn_like(x), alpha=self.noise_std)   # add_instance_noise, train.py:148-149
 
     def step(self, x_s: torch.Tensor, x_t: torch.Tensor):
+        """use_cuda_graph: one graph replay (step_graph).  Otherwise the eager step (step_eager)."""
+        if self.use_cuda_graph:
+            return self.step_graph(x_s, x_t)
+        return self.step_eager(x_s, x_t)
+
+    def step_eager(self, x_s: torch.Tensor, x_t: torch.Tensor):
         model, D = self.model, self.model.D
         # the reference's R1 helper marks the batch as requiring grad (train.py:247); do that to private views so the
         # caller's (possibly reused, in-place refilled) input buffers stay plain tensors
@@ -523,3 +567,99 @@ class IRFDDiscriminatorStep:
                       self.step_count)
         self.last = (loss_real.detach(), loss_fake.detach(), r1.detach())
         return loss.detach()
+
+    # ---------------------------------------------------------------------------------------------- static-graph step
+    def _static_body(self):
+        x_all, out = self._static
+        b = x_all.size(0) // 2
+        model, D = self.model, self.model.D
+        from . import generator
+
+        self.gflat.zero_()
+        for p, v in zip(self.params, self._grad_views):
+            if p.grad is not v:
+                p.grad = v
+        x_s, x_t = x_all[:b].detach(), x_all[b:].detach()
+        with D.native_spectral_norm():
+            d_real_s, d_real_t = D(self._noisy(x_s)), D(self._noisy(x_t))
+            loss_real = 0.5 * (_BCELogitsFn.apply(d_real_s, REAL_LABEL) + _BCELogitsFn.apply(d_real_t, REAL_LABEL))
+            with torch.no_grad():
+                # the G step's Adam rewrote Gd since the last D step: repack its conv weights inside the graph
+                ops.invalidate_packed(self._gd_conv_weights)
+                if _PREPACK:
+                    ops.prepack_conv_weights(generator.synthesis_pack_items(model.Gd.synthesis),
+                                             ops.side_stream(self.device))
+                img, _, _ = model.forward_static_stacked(x_all, self.ctrl)
+            ops.side_stream(self.device).join()
+            d_fake_s, d_fake_t = D(self._noisy(img[:b])), D(self._noisy(img[b:]))
+            loss_fake = 0.5 * (_BCELogitsFn.apply(d_fake_s, FAKE_LABEL) + _BCELogitsFn.apply(d_fake_t, FAKE_LABEL))
+            r1 = 0.5 * (D.r1_penalty(x_s) + D.r1_penalty(x_t))
+        loss = loss_real + loss_fake + self.r1_weight * r1
+        loss.backward()
+        if self.world > 1:   # DDP's gradient average over the ranks (D sits inside the reference's wrapped model)
+            self.buckets.launch(self.gflat)
+            self.buckets.finish()
+        self.step_count += 1
+        ops.adam_step(self.flat, self.gflat, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps,
+                      self.step_count, step_dev=self.step_dev)
+        for o, t in zip(out, (loss, loss_real, loss_fake, r1)):
+            o.copy_(t.detach())
+        # under capture the repacks above were only recorded: eager code must not take them from the pack cache
+        ops.invalidate_packed(self._gd_conv_weights)
+
+    def _load_static(self, x_s, x_t):
+        """Copy the pair into the stacked static batch [x_s; x_t] (allocated, with the 4 loss scalars, on first use)."""
+        if x_s.shape != x_t.shape:
+            raise ops._lib.IrfdError(f"IRFDDiscriminatorStep static step: x_s {tuple(x_s.shape)} and x_t "
+                                     f"{tuple(x_t.shape)} differ; use step_eager")
+        b = x_s.size(0)
+        shape = (2 * b,) + tuple(x_s.shape[1:])
+        if self._static is None or tuple(self._static[0].shape) != shape:
+            self._static = (torch.empty(shape, dtype=torch.float32, device=self.device),
+                            torch.zeros(4, dtype=torch.float32, device=self.device))
+        self._static[0][:b].copy_(x_s, non_blocking=True)
+        self._static[0][b:].copy_(x_t, non_blocking=True)
+
+    def _graph_state(self, x_s):
+        """What a captured graph bakes in besides the buffers it reads: module modes, the batch shape, the encoders'
+        bf16 repacks (keyed by their weights' version counters), style_mixing_prob and the hyper-parameters that are
+        kernel arguments."""
+        m = self.model
+        enc_ver = tuple(e[0].weight._version for e in self.encoders)
+        return (m.training, m.D.training, m.Gd.training, tuple(e.training for e in self.encoders), tuple(x_s.shape),
+                enc_ver, float(m.Gd.style_mixing_prob), float(self.lr), tuple(self.betas), float(self.eps),
+                float(self.r1_weight), float(self.noise_std), self.buckets.enabled)
+
+    def _finish(self):
+        out = self._static[1]
+        self.last = (out[1], out[2], out[3])
+        return out[0]
+
+    def step_graph(self, x_s: torch.Tensor, x_t: torch.Tensor):
+        """One replay of the captured step (captured first, or again when _graph_state changed).  The returned loss
+        and `last` are the graph's static outputs: the next step overwrites them."""
+        key = self._graph_state(x_s)
+        if self.graph is not None and key != self._graph_key:
+            self.graph = None
+        if self.graph is None:
+            self._load_static(x_s, x_t)
+            state = [self.flat, self.m, self.v] + list(self.model.D.buffers())
+            state += [bf for e in self.encoders for bf in e.buffers()]
+            self.graph, self.graph_launches = self._graphed.capture(self, self._static_body, state)
+            self._graph_key = key
+            self.captures += 1
+        self._load_static(x_s, x_t)
+        self._graphed.draw_ctrl()
+        self.graph.replay()
+        self.step_count += 1
+        ops.launch_count += self.graph_launches
+        return self._finish()
+
+    def step_static_eager(self, x_s: torch.Tensor, x_t: torch.Tensor):
+        """The launch sequence of the captured step, launched kernel by kernel: the reference the replay is tested
+        against, and a way to time the step per launch (events cannot be recorded inside a replay)."""
+        self._load_static(x_s, x_t)
+        self._graphed.draw_ctrl()
+        self.step_dev.fill_(self.step_count)
+        self._static_body()
+        return self._finish()
